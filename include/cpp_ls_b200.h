@@ -159,35 +159,26 @@ MRB_API void mrb_als_destroy(mrb_als_problem* p);
 
 /* ------------------------------------------------------------------------------------------
  * 5. Extensions: multi-GPU, one process per GPU (SURVEY.md section 8e).
- *    Users, then movies, are row-partitioned (degree-sorted rows dealt over the ranks, or
- *    nnz-balanced contiguous ranges); each rank holds full replicas of both factor matrices.
- *    The exact-solve kernel (algorithm 4) stores every solved row into all replicas through
- *    NVLink peer pointers, i.e. the all-gather of the factor shards is fused into the producing
- *    kernel; between half-sweeps only a device-side barrier over the same mappings remains.
+ *    The degree-sorted users, then movies, are dealt over the ranks in snake order; each rank
+ *    holds full replicas of both factor matrices.  The exact-solve kernel (algorithm 4) stores
+ *    every solved row into all replicas through NVLink peer pointers, i.e. the all-gather of the
+ *    factor shards is fused into the producing kernel; between half-sweeps only a device-side
+ *    barrier over the same mappings remains.
  * ---------------------------------------------------------------------------------------- */
 
-/* Host-only: bounds[0..world] = first owner of each rank's range, from a CSR pointer array. */
-MRB_API int mrb_shard_ranges(const int* ptr, int owners, int world, int* bounds);
 /* Host-only: the owners rank receives under the dealt partition (degree-sorted owners dealt in
  * snake order), in processing order; out has room for owners / world + 1 entries; returns the count. */
 MRB_API int mrb_dealt_owners(const int* ptr, int owners, int world, int rank, int* out);
-/* Restricts the problem to rank's row ranges and builds its work lists. */
+/* Restricts the problem to the rows dealt to rank and builds its work lists.  The peer replicas
+ * then come from mrb_als_set_peer_pointers (the peer group below sets the shard itself). */
 MRB_API int mrb_als_set_shard(mrb_als_problem* p, int rank, int world);
-/* out4 = {user_lo, user_hi, item_lo, item_hi}. */
-MRB_API int mrb_als_get_shard_ranges(mrb_als_problem* p, int* out4);
-/* Raw device pointers of the two factor matrices (for an NCCL exchange by the caller). */
+/* Raw device pointers of the two factor matrices (this rank's replicas). */
 MRB_API int mrb_als_device_factors(mrb_als_problem* p, void** d_user_factors, void** d_item_factors);
-/* CUDA IPC handles (64 bytes each) of this rank's factor replicas ... */
-MRB_API int mrb_als_ipc_handles(mrb_als_problem* p, unsigned char* user_handle64,
-                                unsigned char* item_handle64);
-/* ... and their counterpart: map every other rank's replicas (handles concatenated by rank). */
-MRB_API int mrb_als_open_peers(mrb_als_problem* p, const unsigned char* user_handles,
-                               const unsigned char* item_handles, int world, int rank);
-/* Same, from device pointers that are already valid in this process (replicas on the same GPU
- * or on peers with access enabled); entry `rank` is ignored. */
+/* The factor replicas of the other ranks, as device pointers that are already valid in this
+ * process (replicas on the same GPU or on peers with access enabled); entry `rank` is ignored. */
 MRB_API int mrb_als_set_peer_pointers(mrb_als_problem* p, void* const* d_user_factor_replicas,
                                       void* const* d_item_factor_replicas, int world);
-/* ---- the peer group of the sharded product path (sharded.ShardedAls, exchange "p2p") --------
+/* ---- the peer group of the sharded path (sharded.ShardedAls) ---------------------------------
  * Creation from a SLICE of the COO: the three pointers address ratings slice_begin ..
  * slice_begin + slice_len - 1 of the num_ratings ratings of the problem; only they cross this
  * rank's host link.  The index build is deferred: exchange the handles, mrb_als_open_peers_all,
@@ -201,11 +192,10 @@ MRB_API int mrb_als_create_slice(const int* user_ids_slice, const int* item_ids_
  * process's barrier words.  An exported block is never returned to the driver (it is recycled by
  * the library's arena), so a mapping a peer has cached can never dangle. */
 MRB_API int mrb_als_ipc_handles_all(mrb_als_problem* p, unsigned char* handles384);
-/* handles_by_rank: world x 384 bytes.  partition 1 deals the degree-sorted rows over the ranks
- * in snake order (the product: rows are stored individually, ownership need not be contiguous);
- * 0 cuts contiguous cost-balanced ranges. */
+/* handles_by_rank: world x 384 bytes.  Maps every other rank's buffers and fixes this rank's
+ * place in the group (its share of the dealt rows). */
 MRB_API int mrb_als_open_peers_all(mrb_als_problem* p, const unsigned char* handles_by_rank,
-                                   int world, int rank, int partition);
+                                   int world, int rank);
 MRB_API int mrb_als_push_coo(mrb_als_problem* p);
 MRB_API int mrb_als_build_index(mrb_als_problem* p);
 /* Device-side barrier over the group (st.release.sys / ld.acquire.sys on the mapped barrier
@@ -224,8 +214,6 @@ MRB_API int mrb_als_upload_factor_rows(mrb_als_problem* p, const double* user_fa
 MRB_API int mrb_als_download_factor_rows(mrb_als_problem* p, double* user_factors,
                                          double* item_factors, int u_lo, int u_hi, int i_lo,
                                          int i_hi, void* stream);
-/* mrb_als_set_shard with the partition made explicit. */
-MRB_API int mrb_als_set_shard_partition(mrb_als_problem* p, int rank, int world, int partition);
 
 /* One exact half-sweep (user_side != 0: users) over this rank's rows, enqueued on `stream`
  * (a cudaStream_t); does not synchronise. */

@@ -93,27 +93,19 @@ def _declare(dll):
     dll.mrb_als_destroy.restype = None
     dll.mrb_als_destroy.argtypes = [c_void_p]
     _B = ctypes.POINTER(ctypes.c_ubyte)
-    dll.mrb_shard_ranges.restype = c_int
-    dll.mrb_shard_ranges.argtypes = [_I, c_int, c_int, _I]
     dll.mrb_dealt_owners.restype = c_int
     dll.mrb_dealt_owners.argtypes = [_I, c_int, c_int, c_int, _I]
     dll.mrb_als_set_shard.restype = c_int
     dll.mrb_als_set_shard.argtypes = [c_void_p, c_int, c_int]
-    dll.mrb_als_get_shard_ranges.restype = c_int
-    dll.mrb_als_get_shard_ranges.argtypes = [c_void_p, _I]
     dll.mrb_als_device_factors.restype = c_int
     dll.mrb_als_device_factors.argtypes = [c_void_p, ctypes.POINTER(c_void_p), ctypes.POINTER(c_void_p)]
-    dll.mrb_als_ipc_handles.restype = c_int
-    dll.mrb_als_ipc_handles.argtypes = [c_void_p, _B, _B]
-    dll.mrb_als_open_peers.restype = c_int
-    dll.mrb_als_open_peers.argtypes = [c_void_p, _B, _B, c_int, c_int]
     dll.mrb_als_set_peer_pointers.restype = c_int
     dll.mrb_als_set_peer_pointers.argtypes = [c_void_p, ctypes.POINTER(c_void_p),
                                               ctypes.POINTER(c_void_p), c_int]
     dll.mrb_als_ipc_handles_all.restype = c_int
     dll.mrb_als_ipc_handles_all.argtypes = [c_void_p, _B]
     dll.mrb_als_open_peers_all.restype = c_int
-    dll.mrb_als_open_peers_all.argtypes = [c_void_p, _B, c_int, c_int, c_int]
+    dll.mrb_als_open_peers_all.argtypes = [c_void_p, _B, c_int, c_int]
     dll.mrb_als_push_coo.restype = c_int
     dll.mrb_als_push_coo.argtypes = [c_void_p]
     dll.mrb_als_build_index.restype = c_int
@@ -129,8 +121,6 @@ def _declare(dll):
     dll.mrb_als_create_slice.restype = c_int
     dll.mrb_als_create_slice.argtypes = [_I, _I, _D, c_int, c_int, c_int, c_int, c_int, c_int,
                                          ctypes.POINTER(c_void_p)]
-    dll.mrb_als_set_shard_partition.restype = c_int
-    dll.mrb_als_set_shard_partition.argtypes = [c_void_p, c_int, c_int, c_int]
     dll.mrb_als_half_sweep.restype = c_int
     dll.mrb_als_half_sweep.argtypes = [c_void_p, c_int, c_void_p]
     dll.mrb_als_stream_sync.restype = c_int

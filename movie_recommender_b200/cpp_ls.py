@@ -259,34 +259,14 @@ class AlsProblem:
 
     # ---- multi-GPU extension (include/cpp_ls_b200.h section 5)
     def set_shard(self, rank, world):
-        """Restrict the problem to this rank's nnz-balanced row ranges (builds the work lists)."""
+        """Restrict the problem to the rows dealt to this rank (builds the work lists)."""
         _lib.check(_dll.mrb_als_set_shard(self._h, rank, world))
-        out = numpy.zeros(4, dtype=numpy.int32)
-        _lib.check(_dll.mrb_als_get_shard_ranges(self._h, _lib.ip(out)))
-        return tuple(int(v) for v in out)   # user_lo, user_hi, item_lo, item_hi
-
-    def shard_ranges(self):
-        out = numpy.zeros(4, dtype=numpy.int32)
-        _lib.check(_dll.mrb_als_get_shard_ranges(self._h, _lib.ip(out)))
-        return tuple(int(v) for v in out)   # user_lo, user_hi, item_lo, item_hi
 
     def device_factors(self):
         """Raw device pointers (user_factors, item_factors)."""
         u, i = ctypes.c_void_p(), ctypes.c_void_p()
         _lib.check(_dll.mrb_als_device_factors(self._h, ctypes.byref(u), ctypes.byref(i)))
         return u.value, i.value
-
-    def ipc_handles(self):
-        hu = (ctypes.c_ubyte * 64)()
-        hi = (ctypes.c_ubyte * 64)()
-        _lib.check(_dll.mrb_als_ipc_handles(self._h, hu, hi))
-        return bytes(hu), bytes(hi)
-
-    def open_peers(self, user_handles, item_handles, rank):
-        world = len(user_handles)
-        bu = (ctypes.c_ubyte * (64 * world)).from_buffer_copy(b"".join(user_handles))
-        bi = (ctypes.c_ubyte * (64 * world)).from_buffer_copy(b"".join(item_handles))
-        _lib.check(_dll.mrb_als_open_peers(self._h, bu, bi, world, rank))
 
     def set_peer_pointers(self, user_ptrs, item_ptrs):
         world = len(user_ptrs)
@@ -300,13 +280,12 @@ class AlsProblem:
         _lib.check(_dll.mrb_als_ipc_handles_all(self._h, h))
         return bytes(h)
 
-    def open_peer_group(self, handles_by_rank, rank, partition=1):
+    def open_peer_group(self, handles_by_rank, rank):
         """Maps every peer's buffers (``handles_by_rank[r]`` = rank r's ``ipc_handles_all()``)
-        and fixes this rank's place in the group; ``partition`` 1 deals the degree-sorted rows
-        over the ranks, 0 cuts contiguous cost-balanced ranges."""
+        and fixes this rank's place in the group (its share of the dealt rows)."""
         world = len(handles_by_rank)
         buf = (ctypes.c_ubyte * (384 * world)).from_buffer_copy(b"".join(handles_by_rank))
-        _lib.check(_dll.mrb_als_open_peers_all(self._h, buf, world, rank, partition))
+        _lib.check(_dll.mrb_als_open_peers_all(self._h, buf, world, rank))
 
     def push_coo(self):
         _lib.check(_dll.mrb_als_push_coo(self._h))
@@ -344,9 +323,6 @@ class AlsProblem:
                                                      ctypes.c_void_p(stream)))
         self._pending_factors = None
 
-    def set_shard_partition(self, rank, world, partition):
-        _lib.check(_dll.mrb_als_set_shard_partition(self._h, rank, world, partition))
-
     def half_sweep(self, user_side, stream):
         _lib.check(_dll.mrb_als_half_sweep(self._h, 1 if user_side else 0, ctypes.c_void_p(stream)))
 
@@ -360,14 +336,6 @@ class AlsProblem:
         out = ctypes.c_float(0)
         _lib.check(_dll.mrb_als_collect_gram_ms(self._h, ctypes.byref(out)))
         return out.value
-
-
-def shard_ranges(ptr, world):
-    """nnz-balanced contiguous row ranges (host only): bounds[0..world] from a CSR pointer array."""
-    ptr = numpy.ascontiguousarray(ptr, dtype=numpy.int32)
-    bounds = numpy.zeros(world + 1, dtype=numpy.int32)
-    _lib.check(_dll.mrb_shard_ranges(_lib.ip(ptr), len(ptr) - 1, world, _lib.ip(bounds)))
-    return bounds
 
 
 def dealt_owners(ptr, rank, world):

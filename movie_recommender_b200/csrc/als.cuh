@@ -32,8 +32,6 @@ struct AlsRunInfo {
     int kernel_launches = 0;   // kernels launched by the sweep loop
 };
 
-// bounds[0..world]: nnz-balanced contiguous owner ranges from a CSR pointer array (host).
-void balanced_ranges(const int* ptr, int owners, int world, int* bounds);
 // Host mirror of the dealt partition: writes rank's owners (processing order), returns the count.
 int dealt_owners_host(const int* ptr, int owners, int world, int rank, int* out);
 
@@ -81,15 +79,12 @@ public:
     // Runs the sweep loop of matrix.cpp:814-890 on the device-resident problem.
     AlsRunInfo run(int algorithm, double min_r_decrease, int max_iteration, int thread_count);
 
-    // ---- multi-GPU (SURVEY.md 8e): users, then movies, are row-partitioned in nnz-balanced
-    // contiguous ranges over `world` ranks; every rank keeps full replicas of both factor
-    // matrices.  The solve kernel stores each solved row into EVERY replica (peer pointers over
-    // NVLink), so the all-gather of the factor shards is fused into the producing kernel.
-    // partition 0: contiguous ranges of equal cost (needed by an NCCL range exchange);
-    // partition 1: the degree-sorted owner list dealt over the ranks in snake order (rows are
-    // stored individually into every replica, so ownership need not be contiguous)
-    void set_shard(int rank, int world, int partition = 0);
-    void shard_ranges(int* user_lo, int* user_hi, int* item_lo, int* item_hi) const;
+    // ---- multi-GPU (SURVEY.md 8e): the degree-sorted users, then movies, are dealt over the
+    // `world` ranks in snake order; every rank keeps full replicas of both factor matrices.  The
+    // solve kernel stores each solved row into EVERY replica (peer pointers over NVLink), so the
+    // all-gather of the factor shards is fused into the producing kernel (rows are stored
+    // individually, so ownership need not be contiguous).
+    void set_shard(int rank, int world);
     // peer replicas of the factor matrices, index = rank (entry `rank` may be the local buffer)
     void set_peers(const std::vector<double*>& user_factor_peers,
                    const std::vector<double*>& item_factor_peers);
@@ -138,7 +133,7 @@ private:
     DevBuf<int> user_ids_, item_ids_, u_ptr_, u_idx_, i_ptr_, i_idx_;
     DevBuf<double> ratings_, uf_, itf_, rmb_;
     float index_ms_ = 0;
-    int rank_ = 0, world_ = 1, partition_ = 0;
+    int rank_ = 0, world_ = 1;
     int slice_begin_ = 0, slice_len_ = -1;
     bool index_built_ = false, pointers_built_ = false, ids_checked_ = false;
     std::vector<int*> uid_peers_, iid_peers_;

@@ -574,25 +574,6 @@ __global__ void k_gather_grouped(const int* __restrict__ idx, const int* __restr
 
 }  // namespace
 
-// bounds[r] = first owner of rank r: contiguous ranges of equal COST, where a row costs its
-// ratings plus a constant for its solve (measured at rank 50: the Cholesky epilogue of one row
-// takes as long as accumulating ~100 ratings, profiles/ncu_k_gram_C3_r01_v3.txt).
-void balanced_ranges(const int* ptr, int owners, int world, int* bounds) {
-    constexpr long long kRowCost = 100;
-    auto cost_before = [&](int o) { return static_cast<long long>(ptr[o]) + kRowCost * o; };
-    const long long total = cost_before(owners);
-    bounds[0] = 0;
-    int o = 0;
-    for (int r = 1; r < world; r++) {
-        const long long target = total * r / world;
-        while (o < owners && cost_before(o) < target) o++;
-        // the boundary nearest to the target (never before the previous boundary)
-        if (o > bounds[r - 1] && target - cost_before(o - 1) < cost_before(o) - target) o--;
-        bounds[r] = o;
-    }
-    bounds[world] = owners;
-}
-
 // Host mirror of the dealt partition (k_lpt_keys + stable_group_by + k_deal_order): the owners
 // rank r receives, in its processing order.  Used by the CPU tests of the N > 1 host logic.
 int dealt_owners_host(const int* ptr, int owners, int world, int rank, int* out) {
@@ -621,7 +602,6 @@ struct Side {
     int n_work = 0;
     int n_multi = 0;
     int n_slots = 0;
-    int lo = 0, hi = 0;   // owner range of this rank
     DevBuf<int> owner_order;   // owners with ratings, longest first (wide-rank path)
     int n_owner_items = 0;
     // where owner o's ratings sit in other_g / rating_g: the CSR pointers of the full grouping,
@@ -699,20 +679,20 @@ __global__ void k_mark_owned(const int* __restrict__ ptr, const int* __restrict_
 }
 
 // ---- work lists, built on the device --------------------------------------------------------
-// Owners of this rank's range in longest-processing-time-first order (degree descending, stable;
-// degrees above 65534 share the first bucket), every owner cut into segments of GRAM_SEG ratings.
+// Owners in longest-processing-time-first order (degree descending, stable; degrees above 65534
+// share the first bucket), every owner cut into segments of GRAM_SEG ratings.
 constexpr int LPT_KEYS = 65536;
 
-__global__ void k_lpt_keys(const int* __restrict__ ptr, int lo, int m, int* __restrict__ key) {
+__global__ void k_lpt_keys(const int* __restrict__ ptr, int m, int* __restrict__ key) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= m) return;
-    const int deg = ptr[lo + i + 1] - ptr[lo + i];
+    const int deg = ptr[i + 1] - ptr[i];
     key[i] = deg >= LPT_KEYS - 1 ? 0 : LPT_KEYS - 1 - deg;
 }
 
 // per owner in LPT order: work items, multi-segment flag, partial-tile slots, non-empty flag
 // (entry m of each array is 0, so that the exclusive scans leave the totals there)
-__global__ void k_owner_counts(const int* __restrict__ ptr, int lo, int m,
+__global__ void k_owner_counts(const int* __restrict__ ptr, int m,
                                const int* __restrict__ order, int* __restrict__ n_items,
                                int* __restrict__ is_multi, int* __restrict__ n_slots,
                                int* __restrict__ nonempty) {
@@ -720,7 +700,7 @@ __global__ void k_owner_counts(const int* __restrict__ ptr, int lo, int m,
     if (j > m) return;
     int nseg = 0;
     if (j < m) {
-        const int o = lo + order[j];
+        const int o = order[j];
         const int deg = ptr[o + 1] - ptr[o];
         nseg = (deg + GRAM_SEG - 1) / GRAM_SEG;
     }
@@ -730,14 +710,14 @@ __global__ void k_owner_counts(const int* __restrict__ ptr, int lo, int m,
     nonempty[j] = nseg > 0;
 }
 
-__global__ void k_write_work(const int* __restrict__ ptr, int lo, int m,
+__global__ void k_write_work(const int* __restrict__ ptr, int m,
                              const int* __restrict__ order, const int* __restrict__ item_at,
                              const int* __restrict__ multi_at, const int* __restrict__ slot_at,
                              const int* __restrict__ nonempty_at, WorkItem* __restrict__ work,
                              int* __restrict__ owner_order) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= m) return;
-    const int o = lo + order[j];
+    const int o = order[j];
     const int beg = ptr[o], end = ptr[o + 1];
     const int nseg = item_at[j + 1] - item_at[j];
     if (nseg == 0) return;   // no equations: the factors keep their previous value
@@ -756,10 +736,6 @@ __global__ void k_write_work(const int* __restrict__ ptr, int lo, int m,
     }
 }
 
-// This rank's owner range and its work lists.  Needs the CSR pointers only, so it is enqueued
-// while the ratings are still on their way to the device.  Host round trips: the pointer array
-// when the rows are sharded (the balanced ranges are a host decision every rank must agree on),
-// and four totals.
 // rank's share of the degree-sorted owner list, dealt in snake order: block t of `world`
 // consecutive owners gives position rank (t even) or world-1-rank (t odd) to this rank, so the
 // per-rank sums of (ratings + solve cost) differ by less than one heavy row
@@ -781,51 +757,36 @@ int dealt_count(int owners, int rank, int world) {
 }
 
 // This rank's owners and its work lists.  Needs the CSR pointers only, so it is enqueued
-// while the ratings are still on their way to the device.  Host round trips: the pointer array
-// when the rows are sharded in contiguous ranges (the balanced ranges are a host decision every
-// rank must agree on), and four totals.
+// while the ratings are still on their way to the device.  Host round trip: the totals.
 void build_side_lists(Side& sd, const int* d_ptr, int owners, int nnz, int rank, int world,
-                      int partition, bool owned_only, cudaStream_t s) {
+                      bool owned_only, cudaStream_t s) {
     PhaseTimer t2("  side: work lists");
-    sd.lo = 0;
-    sd.hi = owners;
     sd.gptr = d_ptr;
     sd.n_grouped = nnz;
-    const bool dealt = world > 1 && partition == 1;
-    MRB_REQUIRE(!owned_only || dealt, "als: owned-rows grouping needs the dealt partition");
+    MRB_REQUIRE(!owned_only || world > 1, "als: owned-rows grouping needs rows dealt over several ranks");
     if (owned_only) {
         sd.cptr.alloc(static_cast<size_t>(owners) + 1);
         MRB_CUDA(cudaMemsetAsync(sd.cptr.p, 0, sizeof(int) * (static_cast<size_t>(owners) + 1), s));
         sd.gptr = sd.cptr.p;
         sd.n_grouped = 0;
     }
-    if (world > 1 && !dealt) {
-        std::vector<int> ptr(static_cast<size_t>(owners) + 1);
-        MRB_CUDA(cudaMemcpyAsync(ptr.data(), d_ptr, sizeof(int) * ptr.size(), cudaMemcpyDeviceToHost, s));
-        MRB_CUDA(cudaStreamSynchronize(s));
-        std::vector<int> bounds(static_cast<size_t>(world) + 1);
-        balanced_ranges(ptr.data(), owners, world, bounds.data());
-        sd.lo = bounds[rank];
-        sd.hi = bounds[rank + 1];
-    }
-    const int m_all = sd.hi - sd.lo;                       // owners that are sorted by degree
-    const int m = dealt ? dealt_count(owners, rank, world) : m_all;   // owners of this rank
+    const int m = dealt_count(owners, rank, world);   // owners of this rank
     sd.n_work = sd.n_multi = sd.n_slots = sd.n_owner_items = 0;
     sd.owner_order.alloc(static_cast<size_t>(std::max(m, 1)));
     // every owner has at most deg / GRAM_SEG + 1 items
     sd.work.alloc(static_cast<size_t>(m) + static_cast<size_t>(nnz) / GRAM_SEG + 1);
     if (m == 0) return;   // (owned-rows mode: cptr is all zero, nothing is grouped)
-    DevBuf<int> key(m_all), kptr(LPT_KEYS + 1), order(m_all), mine;
+    DevBuf<int> key(owners), kptr(LPT_KEYS + 1), order(owners), mine;
     DevBuf<int> counts(4 * (static_cast<size_t>(m) + 1));
     int* item_at = counts.p;
     int* multi_at = item_at + m + 1;
     int* slot_at = multi_at + m + 1;
     int* nonempty_at = slot_at + m + 1;
-    k_lpt_keys<<<ceil_div(m_all, 256), 256, 0, s>>>(d_ptr, sd.lo, m_all, key.p);
+    k_lpt_keys<<<ceil_div(owners, 256), 256, 0, s>>>(d_ptr, owners, key.p);
     MRB_LAUNCHED(1);
-    stable_group_by(key.p, m_all, LPT_KEYS, kptr.p, order.p, s);
+    stable_group_by(key.p, owners, LPT_KEYS, kptr.p, order.p, s);
     const int* my_order = order.p;
-    if (dealt) {
+    if (world > 1) {
         mine.alloc(m);
         k_deal_order<<<ceil_div(m, 256), 256, 0, s>>>(order.p, owners, rank, world, m, mine.p);
         MRB_LAUNCHED(1);
@@ -836,14 +797,14 @@ void build_side_lists(Side& sd, const int* d_ptr, int owners, int nnz, int rank,
         exclusive_scan_i32(sd.cptr.p, sd.cptr.p, static_cast<long long>(owners) + 1, s);
     }
     const int* gptr = sd.gptr;
-    k_owner_counts<<<ceil_div(m + 1, 256), 256, 0, s>>>(gptr, sd.lo, m, my_order, item_at, multi_at,
+    k_owner_counts<<<ceil_div(m + 1, 256), 256, 0, s>>>(gptr, m, my_order, item_at, multi_at,
                                                        slot_at, nonempty_at);
     MRB_LAUNCHED(1);
     exclusive_scan_i32(item_at, item_at, m + 1, s);
     exclusive_scan_i32(multi_at, multi_at, m + 1, s);
     exclusive_scan_i32(slot_at, slot_at, m + 1, s);
     exclusive_scan_i32(nonempty_at, nonempty_at, m + 1, s);
-    k_write_work<<<ceil_div(m, 256), 256, 0, s>>>(gptr, sd.lo, m, my_order, item_at, multi_at,
+    k_write_work<<<ceil_div(m, 256), 256, 0, s>>>(gptr, m, my_order, item_at, multi_at,
                                                  slot_at, nonempty_at, sd.work.p, sd.owner_order.p);
     MRB_LAUNCHED(1);
     MRB_CUDA(cudaGetLastError());
@@ -993,6 +954,15 @@ void launch_wide(const GramArgs& a, bool user_side, int sms, cudaStream_t s) {
         }
     }
 }
+
+// The replicas a solved row is stored into besides the local one: every rank's but this one's.
+template <class Args>
+void set_peer_targets(Args& a, const std::vector<double*>& peers, int rank) {
+    a.n_peers = 0;
+    for (size_t j = 0; j < peers.size(); j++)
+        if (static_cast<int>(j) != rank && peers[j] != nullptr && a.n_peers < 8)
+            a.x_peers[a.n_peers++] = peers[j];
+}
 }  // namespace
 
 struct AlsProblem::GramState {
@@ -1003,7 +973,7 @@ struct AlsProblem::GramState {
     DevBuf<double> sse_owner;  // per-item residual sum of squares from the factorisation
     int sms = 148;
     int st_doubles = 0;
-    int built_rank = -1, built_world = -1, built_partition = -1;
+    int built_rank = -1, built_world = -1;
     int per_sm_block_u = 0, per_sm_block_i = 0;   // occupancy of k_gram_block on this device
     // wide ranks (k > 54): per-batch stored matrices of the block-Gram + shared-memory Cholesky path
     bool wide = false, wide_fused = false;
@@ -1018,11 +988,10 @@ void AlsProblem::ensure_gram() {
     const int n_u = k_ + 1;
     const int m8 = (n_u + 1 + 7) / 8;
     MRB_REQUIRE(n_u <= 160, "als algorithm 3/4: rank above 159 is not supported");
-    if (gram_ && gram_->built_rank == rank_ && gram_->built_world == world_ &&
-        gram_->built_partition == partition_) return;
+    if (gram_ && gram_->built_rank == rank_ && gram_->built_world == world_) return;
     // rows dealt over several GPUs: only the rows this rank owns are grouped (1/world of the
     // sorting work and of the grouped copies); the row pointers of all rows come from histograms
-    const bool owned_only = world_ > 1 && partition_ == 1 && std::getenv("MRB_FULL_INDEX") == nullptr;
+    const bool owned_only = world_ > 1 && std::getenv("MRB_FULL_INDEX") == nullptr;
     if (owned_only) build_pointers(); else build_index();
     PhaseTimer t_g("ensure_gram (work lists)");
     gram_ = std::make_shared<GramState>();
@@ -1030,8 +999,8 @@ void AlsProblem::ensure_gram() {
     int dev = 0;
     MRB_CUDA(cudaGetDevice(&dev));
     MRB_CUDA(cudaDeviceGetAttribute(&g.sms, cudaDevAttrMultiProcessorCount, dev));
-    build_side_lists(g.user, u_ptr_.p, nu_, nnz_, rank_, world_, partition_, owned_only, s_);
-    build_side_lists(g.item, i_ptr_.p, ni_, nnz_, rank_, world_, partition_, owned_only, s_);
+    build_side_lists(g.user, u_ptr_.p, nu_, nnz_, rank_, world_, owned_only, s_);
+    build_side_lists(g.item, i_ptr_.p, ni_, nnz_, rank_, world_, owned_only, s_);
     wait_ratings();
     if (owned_only) {
         build_side_gather_owned(g.user, user_ids_.p, item_ids_.p, ratings_.p, nnz_, nu_, s_);
@@ -1064,7 +1033,6 @@ void AlsProblem::ensure_gram() {
     g.sse_owner.alloc(static_cast<size_t>(std::max(ni_, 1)));
     g.built_rank = rank_;
     g.built_world = world_;
-    g.built_partition = partition_;
 }
 
 // One k_gram launch (algorithm 4) over this rank's rows of one side, timed by a pair of events.
@@ -1090,11 +1058,7 @@ void AlsProblem::launch_half(bool user_side, cudaStream_t stream, int epilogue) 
         a.seg_done = g.counters.p + 1;
         a.debug_skip_solve = std::getenv("MRB_DEBUG_SKIP_SOLVE") != nullptr
                                  ? std::atoi(std::getenv("MRB_DEBUG_SKIP_SOLVE")) : 0;
-        a.n_peers = 0;
-        const std::vector<double*>& peers = user_side ? uf_peers_ : itf_peers_;
-        for (size_t j = 0; j < peers.size(); j++)
-            if (static_cast<int>(j) != rank_ && peers[j] != nullptr && a.n_peers < 8)
-                a.x_peers[a.n_peers++] = peers[j];
+        set_peer_targets(a, user_side ? uf_peers_ : itf_peers_, rank_);
         if (!user_side) {
             MRB_CUDA(cudaMemsetAsync(g.sse_owner.p, 0, sizeof(double) * g.sse_owner.n, stream));
             a.sse_out = g.sse_owner.p;
@@ -1134,11 +1098,7 @@ void AlsProblem::launch_half(bool user_side, cudaStream_t stream, int epilogue) 
         CholArgs c{};
         c.n = n;
         c.x = user_side ? uf_.p : itf_.p;
-        c.n_peers = 0;
-        const std::vector<double*>& peers = user_side ? uf_peers_ : itf_peers_;
-        for (size_t j = 0; j < peers.size(); j++)
-            if (static_cast<int>(j) != rank_ && peers[j] != nullptr && c.n_peers < 8)
-                c.x_peers[c.n_peers++] = peers[j];
+        set_peer_targets(c, user_side ? uf_peers_ : itf_peers_, rank_);
         if (!user_side) {
             MRB_CUDA(cudaMemsetAsync(g.sse_owner.p, 0, sizeof(double) * g.sse_owner.n, stream));
             c.sse_out = g.sse_owner.p;
@@ -1214,11 +1174,7 @@ void AlsProblem::launch_half(bool user_side, cudaStream_t stream, int epilogue) 
                              ? std::atoi(std::getenv("MRB_DEBUG_SKIP_SOLVE")) : 0;
     a.order_mode = std::getenv("MRB_WORK_ORDER") != nullptr ? std::atoi(std::getenv("MRB_WORK_ORDER"))
                                                             : GRAM_DEFAULT_ORDER;
-    a.n_peers = 0;
-    const std::vector<double*>& peers = user_side ? uf_peers_ : itf_peers_;
-    for (size_t j = 0; j < peers.size(); j++)
-        if (static_cast<int>(j) != rank_ && peers[j] != nullptr && a.n_peers < 8)
-            a.x_peers[a.n_peers++] = peers[j];
+    set_peer_targets(a, user_side ? uf_peers_ : itf_peers_, rank_);
     if (!user_side) {
         // every rating belongs to exactly one item, so the per-item residuals of the item
         // half-sweep add up to the training SSE after the sweep -- for free
@@ -1268,20 +1224,10 @@ float AlsProblem::collect_gram_ms() {
     return total;
 }
 
-void AlsProblem::set_shard(int rank, int world, int partition) {
+void AlsProblem::set_shard(int rank, int world) {
     MRB_REQUIRE(world >= 1 && world <= 8 && rank >= 0 && rank < world, "als: bad shard (rank, world)");
-    MRB_REQUIRE(partition == 0 || partition == 1, "als: partition must be 0 (ranges) or 1 (dealt)");
     rank_ = rank;
     world_ = world;
-    partition_ = partition;
-}
-
-void AlsProblem::shard_ranges(int* user_lo, int* user_hi, int* item_lo, int* item_hi) const {
-    MRB_REQUIRE(gram_ != nullptr, "als: shard_ranges before the work lists were built");
-    *user_lo = gram_->user.lo;
-    *user_hi = gram_->user.hi;
-    *item_lo = gram_->item.lo;
-    *item_hi = gram_->item.hi;
 }
 
 void AlsProblem::set_peers(const std::vector<double*>& user_factor_peers,

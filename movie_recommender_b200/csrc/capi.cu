@@ -329,15 +329,6 @@ int mrb_als_run(mrb_als_problem* p, int algorithm, double min_r_decrease, int ma
 
 void mrb_als_destroy(mrb_als_problem* p) { delete p; }
 
-int mrb_shard_ranges(const int* ptr, int owners, int world, int* bounds) {
-    return guarded([&] {
-        MRB_REQUIRE(ptr != nullptr && bounds != nullptr && owners >= 0 && world >= 1,
-                    "mrb_shard_ranges: bad arguments");
-        balanced_ranges(ptr, owners, world, bounds);
-        return 0;
-    });
-}
-
 int mrb_dealt_owners(const int* ptr, int owners, int world, int rank, int* out) {
     return guarded([&] {
         MRB_REQUIRE(ptr != nullptr && out != nullptr && owners >= 0 && world >= 1 && rank >= 0 &&
@@ -357,49 +348,11 @@ int mrb_als_set_shard(mrb_als_problem* p, int rank, int world) {
     });
 }
 
-int mrb_als_get_shard_ranges(mrb_als_problem* p, int* out4) {
-    return guarded([&] {
-        MRB_REQUIRE(p != nullptr && out4 != nullptr, "null argument");
-        p->impl.shard_ranges(&out4[0], &out4[1], &out4[2], &out4[3]);
-        return 0;
-    });
-}
-
 int mrb_als_device_factors(mrb_als_problem* p, void** d_user_factors, void** d_item_factors) {
     return guarded([&] {
         MRB_REQUIRE(p != nullptr, "null problem");
         *d_user_factors = p->impl.user_factors();
         *d_item_factors = p->impl.item_factors();
-        return 0;
-    });
-}
-
-int mrb_als_ipc_handles(mrb_als_problem* p, unsigned char* user_handle64,
-                        unsigned char* item_handle64) {
-    return guarded([&] {
-        MRB_REQUIRE(p != nullptr, "null problem");
-        ipc_export(p->impl.user_factors(), user_handle64);
-        ipc_export(p->impl.item_factors(), item_handle64);
-        return 0;
-    });
-}
-
-int mrb_als_open_peers(mrb_als_problem* p, const unsigned char* user_handles,
-                       const unsigned char* item_handles, int world, int rank) {
-    return guarded([&] {
-        MRB_REQUIRE(p != nullptr && world >= 1 && world <= 8 && rank >= 0 && rank < world,
-                    "mrb_als_open_peers: bad arguments");
-        std::vector<double*> up(world, nullptr), ip(world, nullptr);
-        for (int r = 0; r < world; r++) {
-            if (r == rank) {
-                up[r] = p->impl.user_factors();
-                ip[r] = p->impl.item_factors();
-                continue;
-            }
-            up[r] = static_cast<double*>(ipc_open_cached(user_handles + 64 * r));
-            ip[r] = static_cast<double*>(ipc_open_cached(item_handles + 64 * r));
-        }
-        p->impl.set_peers(up, ip);
         return 0;
     });
 }
@@ -421,7 +374,7 @@ int mrb_als_ipc_handles_all(mrb_als_problem* p, unsigned char* handles /* 6 x 64
 }
 
 int mrb_als_open_peers_all(mrb_als_problem* p, const unsigned char* handles_by_rank, int world,
-                           int rank, int partition) {
+                           int rank) {
     return guarded([&] {
         MRB_REQUIRE(p != nullptr && world >= 1 && world <= PEER_MAX && rank >= 0 && rank < world,
                     "mrb_als_open_peers_all: bad arguments");
@@ -447,7 +400,7 @@ int mrb_als_open_peers_all(mrb_als_problem* p, const unsigned char* handles_by_r
         }
         p->rank = rank;
         p->world = world;
-        p->impl.set_shard(rank, world, partition);   // rank known from here on (pushes skip it)
+        p->impl.set_shard(rank, world);   // rank known from here on (pushes skip it)
         p->impl.set_peers(up, ip);
         p->impl.set_coo_peers(uid, iid, rp);
         return 0;
@@ -527,17 +480,6 @@ int mrb_als_create_slice(const int* user_ids_slice, const int* item_ids_slice,
         MRB_REQUIRE(out != nullptr && slice_len >= 0, "mrb_als_create_slice: bad arguments");
         *out = new mrb_als_problem(user_ids_slice, item_ids_slice, num_ratings, ratings_slice,
                                    num_item_factors, num_users, num_items, slice_begin, slice_len);
-        return 0;
-    });
-}
-
-int mrb_als_set_shard_partition(mrb_als_problem* p, int rank, int world, int partition) {
-    return guarded([&] {
-        MRB_REQUIRE(p != nullptr, "null problem");
-        p->rank = rank;
-        p->world = world;
-        p->impl.set_shard(rank, world, partition);
-        p->impl.half_sweep_prepare();
         return 0;
     });
 }

@@ -44,7 +44,6 @@ def fold_in_users(user_ids, item_ids, ratings, num_users, item_factors, num_item
     with cpp_ls.AlsProblem(user_ids[keep], item_ids[keep], ratings[keep], k, num_users,
                            num_items) as prob:
         prob.set_factors(numpy.zeros(num_users * (k + 1)), item_factors)
-        prob.set_shard(0, 1)
         prob.half_sweep(True, 0)
         user_factors, _ = prob.get_factors_synced()
     user_factors = user_factors.reshape(num_users, k + 1)

@@ -3,32 +3,18 @@ plumbing (rendezvous, the 384-byte handle exchange, max-over-ranks timing), hand
 everything on the data path.
 
 Partitioning: the degree-sorted users, then movies, are dealt over the ``world`` ranks in snake
-order (or cut into contiguous cost-balanced ranges for the NCCL baseline); every rank holds the
-COO and full replicas of both factor matrices, but uploads only its 1/world slice (the slices are
-pushed to the peers over NVLink) and groups only the rows it owns.  Exchange: the one place the
-path shards is the all-gather of the freshly solved factor rows after each half-sweep.  Two
-implementations:
-
-* ``exchange="p2p"`` (default, the product): the solve kernel stores every solved row into all
-  replicas through NVLink peer pointers (CUDA IPC mappings of the other ranks' buffers), i.e. the
-  all-gather is fused into the producing kernel and overlaps the math row by row; between
-  half-sweeps only a device-side flag barrier over the same mappings remains (``csrc/peer.cu``),
-  enqueued on the stream -- no host round trip, no library collective.
-* ``exchange="nccl"`` (the baseline it is compared with): every rank uploads everything, rows are
-  written locally and the contiguous ranges are exchanged with ``torch.distributed.all_gather``
-  on tensors aliasing the library's buffers.
+order; every rank holds the COO and full replicas of both factor matrices, but uploads only its
+1/world slice (the slices are pushed to the peers over NVLink) and groups only the rows it owns.
+Exchange: the one place the path shards is the all-gather of the freshly solved factor rows after
+each half-sweep.  The solve kernel stores every solved row into all replicas through NVLink peer
+pointers (CUDA IPC mappings of the other ranks' buffers), i.e. the all-gather is fused into the
+producing kernel and overlaps the math row by row; between half-sweeps only a device-side flag
+barrier over the same mappings remains (``csrc/peer.cu``), enqueued on the stream -- no host
+round trip, no library collective.
 """
 import numpy as np
 
 from . import cpp_ls
-
-
-class _DevArray:
-    """Wraps a raw device pointer for torch.as_tensor via __cuda_array_interface__."""
-
-    def __init__(self, ptr, n):
-        self.__cuda_array_interface__ = {"shape": (n,), "typestr": "<f8", "data": (ptr, False),
-                                         "version": 3, "strides": None}
 
 
 def io_slice(n, rank, world):
@@ -39,24 +25,20 @@ def io_slice(n, rank, world):
 class ShardedAls:
     """One ALS problem over ``world`` GPUs (this process drives GPU ``rank``).
 
-    ``exchange="p2p"`` (the product).  Host traffic: every rank uploads only its 1/world slice
-    of the COO and of the initial factors and pushes it to the peers over NVLink (copy engines,
-    CUDA IPC mappings), so every byte crosses the box's host memory system once.  Work: the
-    degree-sorted rows are dealt over the ranks (``partition=1``; rows are stored individually
-    into every replica, so ownership need not be contiguous).  Exchange: fused into the solve
-    kernel (peer stores).  Synchronisation: a device-side flag barrier over the same mappings
-    (``peer.cu``), enqueued on the stream -- no host round trip, no library collective on the
-    data path.  ``exchange="nccl"`` is the baseline: full upload per rank, contiguous ranges,
-    ``all_gather`` of the ranges after each half-sweep."""
+    Host traffic: every rank uploads only its 1/world slice of the COO and of the initial factors
+    and pushes it to the peers over NVLink (copy engines, CUDA IPC mappings), so every byte
+    crosses the box's host memory system once.  Work: the degree-sorted rows are dealt over the
+    ranks (rows are stored individually into every replica, so ownership need not be
+    contiguous).  Exchange: fused into the solve kernel (peer stores).  Synchronisation: a
+    device-side flag barrier over the same mappings (``peer.cu``), enqueued on the stream -- no
+    host round trip, no library collective on the data path."""
 
-    def __init__(self, problem, k, num_users, num_items, rank, world, exchange="p2p",
-                 async_upload=False, partition=None, sliced_arrays=False):
+    def __init__(self, problem, k, num_users, num_items, rank, world, sliced_arrays=False):
         import torch
         import torch.distributed as dist
         self.torch, self.dist = torch, dist
         self.rank, self.world, self.k = rank, world, k
         self.nu, self.ni = num_users, num_items
-        self.exchange = exchange
         # sliced_arrays: problem["user_ids" / "item_ids" / "ratings"] are THIS RANK'S slice of a
         # problem of problem["num_ratings_total"] ratings starting at problem["slice_begin"], and
         # problem["user_factors_rows" / "item_factors_rows"] hold just the factor rows of
@@ -64,7 +46,6 @@ class ShardedAls:
         # (config 5: 16 GB of ratings, 10 GB of user factors)
         self.sliced_arrays = sliced_arrays
         self.nnz = int(problem["num_ratings_total"]) if sliced_arrays else len(problem["ratings"])
-        self.partition = (1 if exchange == "p2p" else 0) if partition is None else partition
         import os
         import time
         marks = [("start", time.time())]
@@ -72,70 +53,46 @@ class ShardedAls:
         self.u_rows = io_slice(num_users, rank, world)
         self.i_rows = io_slice(num_items, rank, world)
         if sliced_arrays:
-            if exchange != "p2p":
-                raise ValueError("sliced host arrays need the peer-to-peer path")
             self.u_rows, self.i_rows = tuple(problem["user_rows"]), tuple(problem["item_rows"])
-        if exchange == "p2p":
-            # the device-side barriers below spin (with a 10 s timeout) until every rank has
-            # arrived: enter the construction together, however long each rank's host-side
-            # preparation took
-            if world > 1:
-                dist.barrier()
-            if sliced_arrays:
-                b = int(problem["slice_begin"])
-                self.prob = cpp_ls.AlsProblem(problem["user_ids"], problem["item_ids"], problem["ratings"],
-                                              k, num_users, num_items,
-                                              coo_slice=(b, b + len(problem["ratings"])), total_ratings=self.nnz)
-            else:
-                self.prob = cpp_ls.AlsProblem(problem["user_ids"], problem["item_ids"], problem["ratings"],
-                                              k, num_users, num_items,
-                                              coo_slice=io_slice(self.nnz, rank, world))
-            marks.append(("create (slice upload enqueued)", time.time()))
-            if world > 1:
-                mine = torch.frombuffer(bytearray(self.prob.ipc_handles_all()), dtype=torch.uint8).to(self.device)
-                allh = torch.empty(384 * world, dtype=torch.uint8, device=self.device)
-                dist.all_gather_into_tensor(allh, mine)
-                allh = bytes(allh.cpu().numpy())
-            else:
-                allh = self.prob.ipc_handles_all()
-            marks.append(("handle exchange", time.time()))
-            self.prob.open_peer_group([allh[384 * r:384 * (r + 1)] for r in range(world)], rank,
-                                      self.partition)
-            marks.append(("open peers", time.time()))
-            self.prob.push_coo()            # own slice -> every peer (NVLink)
-            self.prob.peer_barrier()        # problem stream: every rank's slice is everywhere
-            if sliced_arrays:
-                self.prob.upload_factor_rows(problem["user_factors_rows"], problem["item_factors_rows"],
-                                             *self.u_rows, *self.i_rows, rows_only=True)
-            else:
-                uf0 = problem["user_factors0"].reshape(-1)
-                itf0 = problem["item_factors0"].reshape(-1)
-                self.prob.upload_factor_rows(uf0, itf0, *self.u_rows, *self.i_rows)
-            self.prob.build_index()         # id check, both groupings, this rank's work lists
-            marks.append(("index + work lists", time.time()))
-            # second barrier, on the stream the sweeps use and behind this rank's factor pushes:
-            # past it every replica holds the complete initial factors
-            self.prob.peer_barrier(torch.cuda.current_stream().cuda_stream)
-            self.ranges = None
+        # the device-side barriers below spin (with a 10 s timeout) until every rank has
+        # arrived: enter the construction together, however long each rank's host-side
+        # preparation took
+        if world > 1:
+            dist.barrier()
+        if sliced_arrays:
+            b = int(problem["slice_begin"])
+            self.prob = cpp_ls.AlsProblem(problem["user_ids"], problem["item_ids"], problem["ratings"],
+                                          k, num_users, num_items,
+                                          coo_slice=(b, b + len(problem["ratings"])), total_ratings=self.nnz)
         else:
             self.prob = cpp_ls.AlsProblem(problem["user_ids"], problem["item_ids"], problem["ratings"],
-                                          k, num_users, num_items)
-            marks.append(("problem", time.time()))
-            # async_upload: the factors ride the copy stream behind the ratings (the caller keeps
-            # problem["*_factors0"] alive and untouched until the first get_factors)
-            self.prob.set_factors(problem["user_factors0"], problem["item_factors0"],
-                                  wait=not async_upload)
-            self.prob.set_shard_partition(rank, world, 0)
-            self.ranges = self.prob.shard_ranges()
-            pu, pi = self.prob.device_factors()
-            self.uf = torch.as_tensor(_DevArray(pu, num_users * (k + 1)), device=self.device)
-            self.itf = torch.as_tensor(_DevArray(pi, num_items * k), device=self.device)
-            all_ranges = [None] * world
-            dist.all_gather_object(all_ranges, self.ranges)
-            self.u_views = [self.uf[r[0] * (k + 1):r[1] * (k + 1)] for r in all_ranges]
-            self.i_views = [self.itf[r[2] * k:r[3] * k] for r in all_ranges]
-            self.prob.finish_uploads()
-            dist.barrier()
+                                          k, num_users, num_items,
+                                          coo_slice=io_slice(self.nnz, rank, world))
+        marks.append(("create (slice upload enqueued)", time.time()))
+        if world > 1:
+            mine = torch.frombuffer(bytearray(self.prob.ipc_handles_all()), dtype=torch.uint8).to(self.device)
+            allh = torch.empty(384 * world, dtype=torch.uint8, device=self.device)
+            dist.all_gather_into_tensor(allh, mine)
+            allh = bytes(allh.cpu().numpy())
+        else:
+            allh = self.prob.ipc_handles_all()
+        marks.append(("handle exchange", time.time()))
+        self.prob.open_peer_group([allh[384 * r:384 * (r + 1)] for r in range(world)], rank)
+        marks.append(("open peers", time.time()))
+        self.prob.push_coo()            # own slice -> every peer (NVLink)
+        self.prob.peer_barrier()        # problem stream: every rank's slice is everywhere
+        if sliced_arrays:
+            self.prob.upload_factor_rows(problem["user_factors_rows"], problem["item_factors_rows"],
+                                         *self.u_rows, *self.i_rows, rows_only=True)
+        else:
+            uf0 = problem["user_factors0"].reshape(-1)
+            itf0 = problem["item_factors0"].reshape(-1)
+            self.prob.upload_factor_rows(uf0, itf0, *self.u_rows, *self.i_rows)
+        self.prob.build_index()         # id check, both groupings, this rank's work lists
+        marks.append(("index + work lists", time.time()))
+        # second barrier, on the stream the sweeps use and behind this rank's factor pushes:
+        # past it every replica holds the complete initial factors
+        self.prob.peer_barrier(torch.cuda.current_stream().cuda_stream)
         marks.append(("ready", time.time()))
         if rank == 0 and os.environ.get("MRB_E2E_TIMING"):
             import sys
@@ -145,20 +102,14 @@ class ShardedAls:
     def close(self):
         self.prob.close()
 
-    def _exchange(self, user_side, stream):
-        if self.exchange == "p2p":
-            # rows are already in every replica; wait until every rank's kernel has finished
-            self.prob.peer_barrier(stream)
-        else:
-            views = self.u_views if user_side else self.i_views
-            self.dist.all_gather(views, views[self.rank])
-
     def sweep(self):
         stream = self.torch.cuda.current_stream().cuda_stream
+        # after each half-sweep the solved rows are already in every replica; the barrier waits
+        # until every rank's kernel has finished
         self.prob.half_sweep(True, stream)
-        self._exchange(True, stream)
+        self.prob.peer_barrier(stream)
         self.prob.half_sweep(False, stream)
-        self._exchange(False, stream)
+        self.prob.peer_barrier(stream)
 
     def sse(self):
         """Training sum of squared errors after the last sweep, summed over ranks."""
@@ -232,11 +183,11 @@ class ShardedAls:
         clocks = sampler.stop() if sampler is not None else None
         return dict(device_ms=float(ms[0]), gram_ms=float(ms[1]), wall_ms=wall_ms, clocks=clocks,
                     launches=int(launches) * self.world, user_factors=uf, item_factors=itf,
-                    sse=sse, exchange=self.exchange, ranges=self.ranges,
+                    sse=sse, exchange="p2p",   # peer stores + device barrier, named in bench output
                     per_rank_gram_ms=[round(float(v), 4) for v in per_rank.cpu()])
 
 
-def e2e_steps(problem, k, num_users, num_items, rank, world, steps, exchange="p2p", timing=False):
+def e2e_steps(problem, k, num_users, num_items, rank, world, steps, timing=False):
     """End-to-end time of one sharded sweep from HOST buffers, per step: every rank uploads its
     1/world slice of the ratings and of the factors (pushed on to the peers over NVLink), builds
     the indices and its work lists, runs one sweep and copies its 1/world share of the factor
@@ -256,15 +207,10 @@ def e2e_steps(problem, k, num_users, num_items, rank, world, steps, exchange="p2
         dist.barrier()
         torch.cuda.synchronize()
         t0 = time.time()
-        s = ShardedAls(problem, k, num_users, num_items, rank, world, exchange=exchange,
-                       async_upload=True)
+        s = ShardedAls(problem, k, num_users, num_items, rank, world)
         t1 = time.time()
         s.sweep()
-        if exchange == "p2p":
-            s.download_own_rows(uf_host, itf_host)      # synchronises the stream
-        else:
-            torch.cuda.synchronize()
-            s.prob.get_factors(uf_host, itf_host)
+        s.download_own_rows(uf_host, itf_host)      # synchronises the stream
         t2 = time.time()
         dt = torch.tensor([t2 - t0], dtype=torch.float64, device=s.device)
         dist.all_reduce(dt, op=dist.ReduceOp.MAX)
@@ -276,15 +222,12 @@ def e2e_steps(problem, k, num_users, num_items, rank, world, steps, exchange="p2
         if step > 0:
             times.append(float(dt.item()))
     fbytes = (num_users * (k + 1) + num_items * k) * 8
-    mult = 1 if exchange == "p2p" else world
     return dict(sec_per_step=sum(times) / len(times), steps=len(times),
-                h2d_bytes_per_step=mult * (nnz * 16 + fbytes), d2h_bytes_per_step=mult * fbytes,
+                h2d_bytes_per_step=nnz * 16 + fbytes, d2h_bytes_per_step=fbytes,
                 call="sharded.ShardedAls(host buffers) + one sweep + factor download per step on "
                      "every rank; each rank moves its 1/%d slice of the ratings and factors across "
                      "its host link, slices are exchanged over NVLink (peer copies), index build, "
-                     "work lists and peer mapping exchange included" % world
-                if exchange == "p2p" else
-                "ShardedAls(exchange='nccl'): every rank uploads everything")
+                     "work lists and peer mapping exchange included" % world)
 
 
 # ----------------------------------------------------------------------------------------------

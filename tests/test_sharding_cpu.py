@@ -1,6 +1,6 @@
-"""Host-side logic of the multi-GPU path on CPU: world_size-2 gloo processes agree on row ranges
-that tile the rows and balance the ratings (the data-path kernels need GPUs; the N > 1 GPU run is
-tests/test_gpu_sharded.py / bench.py --gpus N)."""
+"""Host-side logic of the multi-GPU path on CPU: world_size-2 gloo processes draw disjoint,
+cost-balanced shares of the dealt rows that together cover every row (the data-path kernels need
+GPUs; the N > 1 GPU run is tests/test_gpu_sharded.py / bench.py --gpus N)."""
 import os
 import subprocess
 import sys
@@ -21,20 +21,6 @@ rank, world = dist.get_rank(), dist.get_world_size()
 u, i = synth.rating_pairs(3000, 700, 90000, 11, 10, seed=5)
 uptr = np.concatenate([[0], np.cumsum(np.bincount(u, minlength=3000))]).astype(np.int32)
 iptr = np.concatenate([[0], np.cumsum(np.bincount(i, minlength=700))]).astype(np.int32)
-ub, ib = cpp_ls.shard_ranges(uptr, world), cpp_ls.shard_ranges(iptr, world)
-mine = (int(ub[rank]), int(ub[rank + 1]), int(ib[rank]), int(ib[rank + 1]))
-allr = [None] * world
-dist.all_gather_object(allr, mine)
-# ranges tile the rows in rank order
-assert allr[0][0] == 0 and allr[-1][1] == 3000 and allr[0][2] == 0 and allr[-1][3] == 700
-for a, b in zip(allr[:-1], allr[1:]):
-    assert a[1] == b[0] and a[3] == b[2]
-# every rank's share of the cost (ratings + 100 per row for its solve) is within 5 %% of the mean
-for r in allr:
-    cu = (uptr[r[1]] - uptr[r[0]]) + 100 * (r[1] - r[0])
-    ci = (iptr[r[3]] - iptr[r[2]]) + 100 * (r[3] - r[2])
-    assert abs(cu - (90000 + 100 * 3000) / world) < 0.05 * (90000 + 100 * 3000)
-    assert abs(ci - (90000 + 100 * 700) / world) < 0.05 * (90000 + 100 * 700)
 # the product partition: degree-sorted rows dealt in snake order -- the ranks' shares are disjoint,
 # cover every row, and their cost is within 1 %% of the mean
 for ptr, rows, unit in ((uptr, 3000, 100), (iptr, 700, 100)):
@@ -50,11 +36,11 @@ for ptr, rows, unit in ((uptr, 3000, 100), (iptr, 700, 100)):
     assert abs(cost - mean) < 0.01 * mean, (cost, mean)
 dist.barrier()
 dist.destroy_process_group()
-print("rank", rank, "ok", mine)
+print("rank", rank, "ok")
 '''
 
 
-def test_shard_ranges_world2_gloo(tmp_path):
+def test_dealt_owners_world2_gloo(tmp_path):
     script = tmp_path / "worker.py"
     script.write_text(WORKER % ROOT)
     env = dict(os.environ, MASTER_ADDR="127.0.0.1", MASTER_PORT="29517")
@@ -74,16 +60,6 @@ def test_dealt_owners_edge_cases():
     # world 2: blocks [5 3] [0 2] (snake: reversed) [4 1]
     assert [list(cpp_ls.dealt_owners(ptr, r, 2)) for r in range(2)] == [[5, 2, 4], [3, 0, 1]]
     assert list(cpp_ls.dealt_owners(np.zeros(1, dtype=np.int32), 0, 3)) == []
-
-
-def test_shard_ranges_edge_cases():
-    ptr = np.array([0, 5, 5, 9, 20, 21, 40], dtype=np.int32)
-    assert list(cpp_ls.shard_ranges(ptr, 1)) == [0, 6]
-    b = cpp_ls.shard_ranges(ptr, 3)
-    assert b[0] == 0 and b[-1] == 6 and np.all(np.diff(b) >= 0)
-    empty = np.zeros(4, dtype=np.int32)                       # three rows, no ratings
-    assert list(cpp_ls.shard_ranges(empty, 2))[0] == 0
-    assert list(cpp_ls.shard_ranges(np.array([0], dtype=np.int32), 4)) == [0, 0, 0, 0, 0]
 
 
 SIM_WORKER = r'''

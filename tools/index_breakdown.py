@@ -13,7 +13,7 @@ for full in (False, True, False, True):
     if full: os.environ["MRB_FULL_INDEX"] = "1"
     else: os.environ.pop("MRB_FULL_INDEX", None)
     prob = cpp_ls.AlsProblem(p["user_ids"], p["item_ids"], p["ratings"], k, nu, ni, coo_slice=(0, nnz))
-    prob.set_shard_partition(0, world, 1)
+    prob.set_shard(0, world)
     cpp_ls.synchronize() if hasattr(cpp_ls, "synchronize") else None
     prob.finish_uploads() if hasattr(prob, "finish_uploads") else None
     time.sleep(0.05)

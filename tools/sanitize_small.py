@@ -50,7 +50,7 @@ p = synth.als_problem(90, 70, 4000, 7, seed=8, min_degrees=False)
 probs = [cpp_ls.AlsProblem(p["user_ids"], p["item_ids"], p["ratings"], 7, 90, 70) for _ in range(2)]
 for r, pr in enumerate(probs):
     pr.set_factors(p["user_factors0"], p["item_factors0"])
-    pr.set_shard_partition(r, 2, 1)
+    pr.set_shard(r, 2)
 for side in (True, False):
     for pr in probs:
         pr.half_sweep(side, 0)

@@ -24,7 +24,7 @@ prob = cpp_ls.AlsProblem(p["user_ids"], p["item_ids"], p["ratings"], k, nu, ni)
 prob.set_factors(p["user_factors0"], p["item_factors0"])
 out = []
 for rank in sorted({0, W // 2, W - 1}):
-    prob.set_shard_partition(rank, W, 1)
+    prob.set_shard(rank, W)
     res = {}
     for name, side in (("user", True), ("item", False)):
         best = 1e9
