@@ -16,9 +16,12 @@
 //
 // K2b "Cholesky".  The augmented matrix stays in the accumulator fragments (no shared memory,
 // see gram_solve); its Cholesky factor's last row is y = L^-1 g, so forward substitution is free
-// and only L^T x = y remains.  lambda = 0 as in the reference: unknowns the data do not
-// determine (pivot <= 1e-12 of the original diagonal) keep their previous value (the solve is
-// for the correction to the warm start).  Ranks above 54 take the block-wise path further down
+// and only L^T x = y remains.  lambda = 0 as in the reference: an unknown whose computed pivot
+// is <= 1e-12 of the original diagonal keeps its previous value (the solve is for the correction
+// to the warm start).  For an owner with fewer ratings than unknowns only the fit A x = b and
+// finite factors are guaranteed: round-off pivots of its rank-deficient block can clear the
+// threshold, and the unknowns behind them are then moved (gram_solve.cuh).  Ranks above 54 take
+// the block-wise path further down
 // (Gram blocks to HBM, one shared-memory Cholesky per owner).
 //
 // Heavy owners are cut into segments of SEG ratings processed by different warps; the partial

@@ -103,9 +103,14 @@ MRB_DEVICE_INLINE double xor_sum_q(double v) {   // sum over the 4 lanes sharing
 //      tile; the C-fragment -> A/B-fragment conversion is two shuffles per 8x4 chunk).
 // Row n of the factor is y = L^-1 g', so only the back substitution L^T delta = y remains; it is
 // done on the fragments as well.  No shared memory is used.
-// The system solved is the CORRECTION form  G delta = g - G x0,  x = x0 + delta: unknowns whose
-// pivot falls below 1e-12 of the original diagonal get delta = 0 (they keep their previous value,
-// as they do under the reference's warm-started CG), the others are solved consistently.
+// The system solved is the CORRECTION form  G delta = g - G x0,  x = x0 + delta: an unknown whose
+// pivot as COMPUTED falls below 1e-12 of the original diagonal gets delta = 0 and keeps its
+// previous value (as under the reference's warm-started CG); the others are solved consistently
+// around it.  What is guaranteed for an owner with fewer ratings than unknowns is the fit
+// A x = b and finite factors, not which unknowns keep x0: the exact pivots of its rank-deficient
+// block are 0, but their round-off can exceed the threshold (seen at 1e-11 .. 3e-9 of the
+// diagonal when the determined block is ill-conditioned), and such an unknown is then moved --
+// by as much as the data leave it free to, tens of times its start on the emulated warp.
 // ------------------------------------------------------------------------------------------
 // VARIANT 0: pivot columns eliminated over the whole tile column, scalar back substitution.
 // VARIANT 2: an identity tile rides through the pivot loop of every tile column and comes out as

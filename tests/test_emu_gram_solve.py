@@ -11,6 +11,7 @@ import numpy as np
 import pytest
 
 from conftest import ROOT
+from oracle import exact_als
 
 EMU_DIR = os.path.join(ROOT, "tests", "emu")
 
@@ -41,19 +42,26 @@ def emu(request):
     return solve
 
 
-@pytest.mark.parametrize("n,ratings", [(51, 120), (50, 300), (11, 40), (3, 9), (7, 7), (23, 64)])
+@pytest.mark.parametrize("n,ratings", [(51, 120), (50, 300), (11, 40), (3, 9), (7, 7), (23, 64)] +
+                         # every order the solve is instantiated for: all (M8, n mod 8) classes,
+                         # square, one spare rating, well determined
+                         [(n, d) for n in range(1, 56) for d in (n, n + 1, 3 * n + 5)
+                          if (n, d) not in ((3, 9), (7, 7))])
 def test_exact_solve_and_residual(emu, n, ratings):
-    """User side (n = k + 1 with the bias column) and movie side (n = k) shapes, k = 50 included."""
+    """User side (n = k + 1 with the bias column) and movie side (n = k) shapes, k = 50 included;
+    error within the per-owner tolerance of oracle/exact_als.py."""
     rng = np.random.default_rng(n * 1000 + ratings)
     A = rng.uniform(-1, 1, (ratings, n))
     A[:, -1] = 1.0                                   # the bias column of a user row
     b = rng.normal(0, 1, ratings)
     x0 = rng.uniform(-1, 1, n)
     x, sse = emu(A, b, x0)
-    want = np.linalg.lstsq(A, b, rcond=None)[0]
-    assert np.max(np.abs(x - want)) <= 1e-9 * max(1.0, np.max(np.abs(want)))
+    ref = exact_als.solve_owner(A, b, x0)
+    assert ref["determined"]
+    want = ref["x"]
+    assert np.max(np.abs(x - want)) <= min(ref["tol"], 1e-9 * max(1.0, np.max(np.abs(want))))
     r = b - A @ want
-    assert abs(sse - r @ r) <= 1e-9 * max(1.0, b @ b)
+    assert abs(sse - r @ r) <= max(1e-9, ref["tol"]) * max(1.0, b @ b)
 
 
 def test_warm_start_is_a_fixed_point(emu):

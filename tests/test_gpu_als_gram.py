@@ -10,34 +10,9 @@ import pytest
 
 from conftest import bits_equal, load_golden
 from movie_recommender_b200 import synth
+from oracle.exact_als import numpy_half_sweeps
 
 pytestmark = pytest.mark.gpu
-
-
-def numpy_half_sweeps(p, uf, itf, sweeps=1):
-    """Exact ALS: every row's least-squares problem solved with numpy.linalg.lstsq (fp64)."""
-    k, nu, ni = p["k"], p["num_users"], p["num_items"]
-    u, i, r = p["user_ids"], p["item_ids"], p["ratings"]
-    uf = uf.reshape(nu, k + 1).copy()
-    itf = itf.reshape(ni, k).copy()
-    ou = np.argsort(u, kind="stable")
-    oi = np.argsort(i, kind="stable")
-    up = np.concatenate([[0], np.cumsum(np.bincount(u, minlength=nu))])
-    ip = np.concatenate([[0], np.cumsum(np.bincount(i, minlength=ni))])
-    for _ in range(sweeps):
-        for a in range(nu):
-            rows = ou[up[a]:up[a + 1]]
-            if len(rows) == 0:
-                continue
-            A = np.hstack([itf[i[rows]], np.ones((len(rows), 1))])
-            uf[a] = np.linalg.lstsq(A, r[rows], rcond=None)[0]
-        for b in range(ni):
-            rows = oi[ip[b]:ip[b + 1]]
-            if len(rows) == 0:
-                continue
-            A = uf[u[rows], :k]
-            itf[b] = np.linalg.lstsq(A, r[rows] - uf[u[rows], k], rcond=None)[0]
-    return uf.reshape(-1), itf.reshape(-1)
 
 
 def rel_err(a, b):
