@@ -1,4 +1,4 @@
-// Gram-block ALS (algorithm 4: gathered Gram + register-resident Cholesky; algorithm 3: the
+// Gram-block ALS (algorithm 4: gathered Gram + per-warp Cholesky; algorithm 3: the
 // reference's global-scalar CG run on the stored Gram blocks).  See als.cuh for the data layout.
 //
 // K1 "gather-Gram".  Every row r of the reference's materialised user_A touches only user u's
@@ -7,18 +7,19 @@
 //     G_i = sum_{u in U_i} a_u a_u^T,   a_u =  user_factors[u, 0..k-1]            (item side)
 // and A^T b = concat(g_o), g_o = sum b a  with b = rating (user side) or rating - user bias
 // (item side, matrix.cpp:1012-1031).  One warp walks an owner's ratings (CSR for users, CSC for
-// items, both precomputed by K4), gathers the opposite side's factor rows straight from L2/HBM
-// into mma fragments and accumulates the AUGMENTED Gram matrix  sum [a;b][a;b]^T  in fp64 on the
-// tensor cores (mma.sync m8n8k4 f64, SASS DMMA.8x8x4; measured 37.1 TFLOP/s on this B200,
-// vs 33.8 for DFMA -- tools/fp64_peak.cu).  Only the lower-triangular 8x8 tiles are computed.
-// The fragment for 8-wide tile t of ratings q..q+3 is the same register whether it is used as
-// the A operand (row.k) or the B operand (k.col), so one set of loads feeds both.
+// items, both precomputed by K4), gathers the opposite side's factor rows from L2/HBM through a
+// per-warp cp.async ring in shared memory into mma fragments and accumulates the AUGMENTED Gram
+// matrix  sum [a;b][a;b]^T  in fp64 on the tensor cores (mma.sync m8n8k4 f64, SASS DMMA.8x8x4;
+// measured 37.1 TFLOP/s on this B200, vs 33.8 for DFMA -- tools/fp64_peak.cu).  Only the
+// lower-triangular 8x8 tiles are computed.  The fragment for 8-wide tile t of ratings q..q+3 is
+// the same register whether it is used as the A operand (row.k) or the B operand (k.col), so one
+// set of loads feeds both.
 //
-// K2b "Cholesky".  The augmented matrix stays in the accumulator fragments (no shared memory,
-// see gram_solve); its Cholesky factor's last row is y = L^-1 g, so forward substitution is free
-// and only L^T x = y remains.  lambda = 0 as in the reference: an unknown whose computed pivot
-// is <= 1e-12 of the original diagonal keeps its previous value (the solve is for the correction
-// to the warm start).  For an owner with fewer ratings than unknowns only the fit A x = b and
+// K2b "Cholesky".  The accumulator fragments are parked in a per-warp shared-memory slot and
+// factored there tile column by tile column (gram_solve_tiles); the Cholesky factor's last row is
+// y = L^-1 g, so forward substitution is free and only L^T x = y remains.  lambda = 0 as in the
+// reference: an unknown whose computed pivot is <= 1e-12 of the original diagonal keeps its
+// previous value (the solve is for the correction to the warm start).  For an owner with fewer ratings than unknowns only the fit A x = b and
 // finite factors are guaranteed: round-off pivots of its rank-deficient block can clear the
 // threshold, and the unknowns behind them are then moved (gram_solve.cuh).  Ranks above 54 take
 // the block-wise path further down
@@ -44,26 +45,38 @@ namespace {
 
 constexpr int GRAM_SEG = 2048;     // ratings per work item
 constexpr int GRAM_WARPS = 4;      // warps per CTA
+// Three CTAs of four warps per SM -- three warps per scheduler, so that the fp64 tensor pipe stays
+// fed while one of them is in its latency-bound Cholesky chain (one warp alone reaches only ~64 %
+// of the DMMA rate two warps reach).  That caps k_gram at 168 registers: the gather ring and the
+// Gram tiles during the solve live in shared memory, not in registers.
 // (Measured and rejected, profiles/ab_solve_r02.log: one CTA of 8 warps per SM whose two warps
-// per scheduler pass a "tensor token", so that one accumulates while the other solves -- a single
-// warp reaches only 64 % of the accumulation rate two warps reach together: 7.8 vs 6.6 ms.)
-// (Measured and rejected as well, profiles/ab_pair_r02.log: the two warps of a scheduler meeting
-// at a named barrier after their accumulation so that both accumulate and both solve at the same
-// time -- 10.7 vs 9.67 ms.  The solve is NOT slowed by the neighbour's DMMA stream: with the
-// accumulation switched off (MRB_DEBUG_SKIP_SOLVE=4) the user-side solves alone take 2.69 ms,
-// accumulation alone 3.37 ms, together 5.91 ms.  It is an in-order chain of ~3.7 k instructions
-// at ~5.6 cycles each; profiles/lat_fp64_r02.txt has the instruction latencies.)
-// (CTA shapes other than 4 warps leave schedulers unevenly loaded -- warp w of a CTA runs on
-// scheduler w mod 4: 3 CTAs x 3 warps at 224 registers 12.3 ms, 2 x 5 warps at 200 registers
-// 16.4 ms per sweep, profiles/ab_shape_r02.log.)
-template <bool USER>
-constexpr int gram_warps() { return GRAM_WARPS; }
+// per scheduler pass a "tensor token", so that one accumulates while the other solves: 7.8 vs
+// 6.6 ms.  Profiles/ab_pair_r02.log: the two warps of a scheduler meeting at a named barrier after
+// their accumulation so that both accumulate and both solve at the same time -- 10.7 vs 9.67 ms.
+// The solve is an in-order chain of ~3.7 k instructions at ~5.6 cycles each;
+// profiles/lat_fp64_r02.txt has the instruction latencies.  CTA shapes other than 4 warps leave
+// schedulers unevenly loaded -- warp w of a CTA runs on scheduler w mod 4, profiles/ab_shape_r02.log.)
+constexpr int GRAM_CTAS_PER_SM = 3;
+// k-steps of gathered fragments in the ring (RD - 1 in flight ahead of the one being used)
 #ifndef GRAM_RING_USER
-#define GRAM_RING_USER 3           // fragment sets in flight, user half-sweep (gathers hit L2)
+#define GRAM_RING_USER 3           // user half-sweep (gathers hit L2)
 #endif
 #ifndef GRAM_RING_ITEM
 #define GRAM_RING_ITEM 5           // item half-sweep (the user factors spill out of L2)
 #endif
+template <bool USER>
+constexpr int gram_ring() { return USER ? GRAM_RING_USER : GRAM_RING_ITEM; }
+static_assert(GRAM_RING_USER >= 2 && GRAM_RING_ITEM >= 2, "the gather ring needs two stages");
+enum { EPI_SOLVE = 0, EPI_STORE = 1 };
+// shared memory of one warp, in doubles: the ring ([stage][element][lane]: the M8 fragment
+// elements and the rating per lane and k-step), overlapped by the slot the solve parks the ST
+// tiles in ([tile][lane][2])
+template <int M8, bool USER, int EPI>
+constexpr int gram_warp_doubles() {
+    return (EPI == EPI_SOLVE && M8 * (M8 + 1) * 32 > gram_ring<USER>() * (M8 + 1) * 32)
+               ? M8 * (M8 + 1) * 32
+               : gram_ring<USER>() * (M8 + 1) * 32;
+}
 
 #ifndef GRAM_DEFAULT_ORDER
 #define GRAM_DEFAULT_ORDER 0
@@ -85,8 +98,6 @@ __device__ __forceinline__ double aug_elem(const double* __restrict__ row, doubl
     }
     return j <= k ? row[j] : 0.0;
 }
-
-enum { EPI_SOLVE = 0, EPI_STORE = 1 };
 
 // Ticket -> position in the work list (sorted longest first).
 //   0: in list order (longest processing time first);
@@ -110,26 +121,26 @@ __device__ double g_zero_row[176];   // zero-initialised: the factor row of a pa
 #endif
 
 template <int M8, bool USER, int EPI>
-// (no minimum-CTAs argument: naming even the default "1" changes ptxas' schedule of the movie-side
-// kernel -- 4.47 instead of 3.73 ms per launch at C3, profiles/ab_tree_r02.log; forcing 3 CTAs per
-// SM (168 registers, 0.3-0.9 KB of spills) was measured as well: 10.2 / 13.2 ms per sweep vs 9.8)
-#ifdef GRAM_MIN_CTAS
-__global__ void __launch_bounds__(gram_warps<USER>() * 32, GRAM_MIN_CTAS)
-#else
-__global__ void __launch_bounds__(gram_warps<USER>() * 32)
-#endif
+__global__ void __launch_bounds__(GRAM_WARPS * 32, GRAM_CTAS_PER_SM)
 k_gram(const GramArgs A) {
     constexpr int ST = M8 * (M8 + 1) / 2;
+    constexpr int RD = gram_ring<USER>();
+    constexpr int RS = M8 + 1;   // doubles per lane and ring stage: M8 fragment elements, the rating
+    extern __shared__ __align__(16) double gram_smem[];
     const int lane = threadIdx.x & 31;
     const int q = lane & 3, p = lane >> 2;
     const int n = A.n, k = A.k;
+    // this warp's shared memory: the gather ring, [stage][element][lane] (each lane copies and reads
+    // only its own fragment elements: no warp-level synchronisation inside the accumulation, and
+    // lane-contiguous doubles are bank-conflict free), overlapped by the slot the solve parks the
+    // Gram tiles in ([tile][lane][2]) -- the ring is dead during the solve
+    double* const wsm = gram_smem + (threadIdx.x >> 5) * gram_warp_doubles<M8, USER, EPI>();
 
     // Element j = 8 t + p of the augmented row [a; b] (users: a = item factors, 1 for the bias,
     // b = rating; items: a = user factors, b = rating - user bias formed at use time).  The order
     // n + 1 fills the last tile, so k >= 8 (M8 - 1) - 1: every tile before the last two (users) /
     // the last one (items) is a plain load; only the NS special tiles need the per-lane choice,
     // and that choice is fixed for the whole kernel.
-    constexpr int RD = USER ? GRAM_RING_USER : GRAM_RING_ITEM;
     constexpr int PLAIN = USER ? (M8 >= 2 ? M8 - 2 : 0) : M8 - 1;
     constexpr int NS = M8 - PLAIN;
     bool sp_load[NS], sp_one[NS], sp_rating[NS];
@@ -143,12 +154,25 @@ k_gram(const GramArgs A) {
 
     // Dynamic scheduler, one ticket ahead: the atomic for the NEXT work item is issued before the
     // current item's accumulation and its WorkItem is loaded before the current item's epilogue,
-    // so that neither latency is exposed between two owners (only 2 warps share a scheduler).
+    // so that neither latency is exposed between two owners.
     int ticket = 0;
     if (lane == 0) ticket = atomicAdd(A.work_counter, 1);
     int w = __shfl_sync(0xffffffffu, ticket, 0);
     WorkItem wi_next{};
     if (w < A.n_work) wi_next = A.work[work_index(w, A.n_work, A.order_mode)];
+    // ids of the first three 32-rating batches of an owner; the next owner's are requested
+    // before the current owner's solve, so that they land while it is factored
+    int ids_cur = 0, ids_nxt = 0, ids_nx2 = 0;
+    bool ids_ready = false;
+    auto first_batches = [&](const WorkItem& it) {
+        const int c = (A.debug_skip_solve & 4) ? 0 : it.end - it.beg;   // 4 = measurement only: the solve alone
+        ids_cur = ids_nxt = ids_nx2 = 0;
+        if (lane < c) ids_cur = GRAM_LD_ID(A.other_g + it.beg + lane);
+        if (32 + lane < c) ids_nxt = GRAM_LD_ID(A.other_g + it.beg + 32 + lane);
+        // a third batch in flight: with only one batch ahead the k-steps ran into the latency
+        // of the id stream (HBM) every 8 steps (11.2 -> 10.5 ms per sweep at C3)
+        if (64 + lane < c) ids_nx2 = GRAM_LD_ID(A.other_g + it.beg + 64 + lane);
+    };
     for (;;) {
         if (w >= A.n_work) break;
         const WorkItem wi = wi_next;
@@ -171,92 +195,65 @@ k_gram(const GramArgs A) {
 #pragma unroll
         for (int t = 0; t < ST; t++) { acc[t][0] = 0; acc[t][1] = 0; }
 
-        // Fragments are fetched TWO k-steps ahead of their use (f -> f1 -> f2), ids/ratings a
-        // whole 32-rating batch ahead, so that an HBM miss (user factors do not fit L2 entirely)
-        // has ~2 x 28 DMMA issue times to land.
-        const int cnt = (A.debug_skip_solve & 4) ? 0 : wi.end - wi.beg;   // 4 = measurement only: the solve alone
+        // Fragments and ratings are copied into the shared-memory ring RD - 1 k-steps ahead of
+        // their use (cp.async, one commit group per k-step) and read with ld.shared right before
+        // their DMMAs; ids travel a whole 32-rating batch ahead, so that an HBM miss (user
+        // factors do not fit L2 entirely) has ~(RD - 1) x 28 DMMA issue times to land.
+        const int cnt = (A.debug_skip_solve & 4) ? 0 : wi.end - wi.beg;
         const int nsteps = (cnt + 3) >> 2;
-        int ids_cur = 0, ids_nxt = 0;
-        double rts_cur = 0, rts_nxt = 0;
-        if (lane < cnt) { ids_cur = GRAM_LD_ID(A.other_g + wi.beg + lane); rts_cur = GRAM_LD_ID(A.rating_g + wi.beg + lane); }
-        if (32 + lane < cnt) { ids_nxt = GRAM_LD_ID(A.other_g + wi.beg + 32 + lane); rts_nxt = GRAM_LD_ID(A.rating_g + wi.beg + 32 + lane); }
-        // a third batch in flight: with only one batch ahead the k-steps ran into the latency
-        // of the id / rating streams (HBM) every 8 steps (11.2 -> 10.5 ms per sweep at C3)
-        int ids_nx2 = 0;
-        double rts_nx2 = 0;
-        if (64 + lane < cnt) { ids_nx2 = GRAM_LD_ID(A.other_g + wi.beg + 64 + lane); rts_nx2 = GRAM_LD_ID(A.rating_g + wi.beg + 64 + lane); }
-#ifdef GRAM_ID_BATCHES4
-        int ids_nx3 = 0;
-        double rts_nx3 = 0;
-        if (96 + lane < cnt) { ids_nx3 = GRAM_LD_ID(A.other_g + wi.beg + 96 + lane); rts_nx3 = GRAM_LD_ID(A.rating_g + wi.beg + 96 + lane); }
-#endif
-        // prep(st): the row pointer and rating of k-step `st` (ratings 4 st .. 4 st + 3) from the
-        // id batches; st's batch is the current or the next one
-        auto prep = [&](const double*& rowp, double& rt, int st, int batch_of_cur) {
+        if (!ids_ready) first_batches(wi);
+        ids_ready = false;
+        __syncwarp();   // every lane is done with the previous owner's slot, which the ring overlaps
+        // issue(st, batch_of_cur, dst): copy this lane's fragment elements of k-step `st` (ratings
+        // 4 st .. 4 st + 3; its batch is the current or the next one) and the rating of its row
+        // to dst.  Padding ratings copy zeros; the special tiles copy the raw element where there
+        // is one, the 1 / rating / rating - bias choice is made when the fragment is USED
+        auto issue = [&](int st, int batch_of_cur, double* dst) {
             const bool from_next = (st >> 3) != batch_of_cur;
             const int src = ((st & 7) << 2) + q;
             int id = __shfl_sync(0xffffffffu, from_next ? ids_nxt : ids_cur, src);
             if (A.debug_skip_solve & 2) id &= 15;   // measurement only: every gather hits L1
-            rt = shfl_double(from_next ? rts_nxt : rts_cur, src);   // 0 past the end
             const bool valid = (st << 2) + q < cnt;
             // the padding ratings of the last k-step read a row of zeros: no per-element select
-            rowp = (valid ? A.other_f + static_cast<size_t>(id) * A.other_stride : g_zero_row) + p;
-        };
-        // loads(dst, rowp): request the fragments.  Special tiles get the raw load only (or 0);
-        // the 1 / rating / rating - bias choice is made when the fragment is USED, two k-steps
-        // later: an instruction that consumes a value just requested from memory would stall
-        // the warp for the whole latency
-        auto loads = [&](double (&dst)[M8], const double* rowp) {
+            const double* rowp = (valid ? A.other_f + static_cast<size_t>(id) * A.other_stride : g_zero_row) + p;
 #pragma unroll
-            for (int t = 0; t < PLAIN; t++) dst[t] = rowp[8 * t];
+            for (int t = 0; t < PLAIN; t++) cp_async8(dst + t * 32, rowp + 8 * t);
 #pragma unroll
-            for (int s = 0; s < NS; s++) {
-                double v = 0.0;
-                if (sp_load[s]) v = rowp[8 * (PLAIN + s)];
-                dst[PLAIN + s] = v;
-            }
+            for (int s = 0; s < NS; s++)
+                if (sp_load[s]) cp_async8(dst + (PLAIN + s) * 32, rowp + 8 * (PLAIN + s));
+            cp_async8(dst + M8 * 32, valid ? A.rating_g + wi.beg + (st << 2) + q : g_zero_row);
         };
-        const double* rowp_pend;   // pointer / rating of the next k-step to be requested
-        double rt_pend;
         const bool bias_lane = !USER && p == (k & 7);   // index k lives in the last tile (k>>3 == M8-1)
-        // one k-step: refill the id batch, request the fragments of step + RD - 1 into `fn`,
-        // resolve the special elements of `fu` (requested RD - 1 steps ago), issue the 28 DMMAs
-        auto kstep = [&](double (&fu)[M8], double rtu, double (&fn)[M8], double& rtn, int step) {
+        // one k-step: refill the id batch, request the fragments of step + RD - 1 into ring slot
+        // `rn`, wait for those of `step` (slot `ru`), resolve their special elements, 28 DMMAs
+        auto kstep = [&](int step, int ru, int rn) {
             if ((step & 7) == 0 && step > 0) {
                 ids_cur = ids_nxt;
-                rts_cur = rts_nxt;
                 ids_nxt = ids_nx2;
-                rts_nxt = rts_nx2;
-#ifdef GRAM_ID_BATCHES4
-                ids_nx2 = ids_nx3;
-                rts_nx2 = rts_nx3;
-                const int e = (step << 2) + 96 + lane;
-                ids_nx3 = 0;
-                rts_nx3 = 0;
-                if (e < cnt) { ids_nx3 = GRAM_LD_ID(A.other_g + wi.beg + e); rts_nx3 = GRAM_LD_ID(A.rating_g + wi.beg + e); }
-#else
                 const int e = (step << 2) + 64 + lane;
                 ids_nx2 = 0;
-                rts_nx2 = 0;
-                if (e < cnt) { ids_nx2 = GRAM_LD_ID(A.other_g + wi.beg + e); rts_nx2 = GRAM_LD_ID(A.rating_g + wi.beg + e); }
-#endif
+                if (e < cnt) ids_nx2 = GRAM_LD_ID(A.other_g + wi.beg + e);
             }
-            if (step + RD - 1 < nsteps) {
-                prep(rowp_pend, rt_pend, step + RD - 1, step >> 3);
-                loads(fn, rowp_pend);
-                rtn = rt_pend;
-            }
+            if (step + RD - 1 < nsteps) issue(step + RD - 1, step >> 3, wsm + rn * (RS * 32) + lane);
+            cp_async_commit_group();   // (possibly empty: keeps the group count in step)
+            cp_async_wait_group<RD - 1>();   // this lane's copies of k-step `step` have landed
+            const double* fs = wsm + ru * (RS * 32) + lane;
+            double fu[M8];
+#pragma unroll
+            for (int t = 0; t < PLAIN; t++) fu[t] = fs[t * 32];
+            const double rtu = fs[M8 * 32];   // 0 past the end
             if (USER) {
                 const double one = (step << 2) + q < cnt ? 1.0 : 0.0;   // padding ratings are all-zero
 #pragma unroll
                 for (int s = 0; s < NS; s++) {
-                    double v = fu[PLAIN + s];
+                    double v = sp_load[s] ? fs[(PLAIN + s) * 32] : 0.0;
                     v = sp_one[s] ? one : v;
                     v = sp_rating[s] ? rtu : v;
                     fu[PLAIN + s] = v;
                 }
-            } else if (bias_lane) {
-                fu[M8 - 1] = rtu - fu[M8 - 1];   // b = rating - user bias (matrix.cpp:1029)
+            } else {
+                const double v = sp_load[0] ? fs[(M8 - 1) * 32] : 0.0;
+                fu[M8 - 1] = bias_lane ? rtu - v : v;   // b = rating - user bias (matrix.cpp:1029)
             }
 #pragma unroll
             for (int ti = 0; ti < M8; ti++)
@@ -264,40 +261,37 @@ k_gram(const GramArgs A) {
                 for (int tj = 0; tj <= ti; tj++)
                     dmma884(acc[TI(ti, tj)][0], acc[TI(ti, tj)][1], fu[ti], fu[tj]);
         };
-        // a static ring of RD fragment sets (no register moves between steps); fragments are
-        // requested RD - 1 k-steps before their use
-        double fr[RD][M8], rtr[RD];
 #pragma unroll
         for (int r = 0; r < RD - 1; r++) {
-            prep(rowp_pend, rt_pend, r, 0);
-            loads(fr[r], rowp_pend);
-            rtr[r] = rt_pend;
+            if (r < nsteps) issue(r, 0, wsm + r * (RS * 32) + lane);
+            cp_async_commit_group();
         }
-        rtr[RD - 1] = 0;
+        // the ring slots rotate statically: k-step step + r uses slot r
         for (int step = 0; step < nsteps; step += RD) {
 #pragma unroll
             for (int r = 0; r < RD; r++)
-                if (r == 0 || step + r < nsteps)
-                    kstep(fr[r], rtr[r], fr[(r + RD - 1) % RD], rtr[(r + RD - 1) % RD], step + r);
+                if (r == 0 || step + r < nsteps) kstep(step + r, r, (r + RD - 1) % RD);
         }
 
         // ---------------- multi-segment owners: ordered reduction by the last arriver --------
         if (wi.nseg > 1) {
-            double* mine = A.partials + (static_cast<size_t>(wi.slot) + wi.seg) * (ST * 64);
+            // (the segment fields are loaded only here: one register each less across the loop)
+            const WorkItem wm = A.work[work_index(w, A.n_work, A.order_mode)];
+            double* mine = A.partials + (static_cast<size_t>(wm.slot) + wm.seg) * (ST * 64);
 #pragma unroll
             for (int t = 0; t < ST; t++)
                 *reinterpret_cast<double2*>(mine + (t * 32 + lane) * 2) = make_double2(acc[t][0], acc[t][1]);
             __threadfence();
             __syncwarp();
             int arrived = 0;
-            if (lane == 0) arrived = atomicAdd(A.seg_done + wi.multi, 1);
+            if (lane == 0) arrived = atomicAdd(A.seg_done + wm.multi, 1);
             arrived = __shfl_sync(0xffffffffu, arrived, 0);
-            if (arrived != wi.nseg - 1) { advance(); continue; }   // someone else finishes this owner
+            if (arrived != wm.nseg - 1) { advance(); continue; }   // someone else finishes this owner
             __threadfence();
 #pragma unroll
             for (int t = 0; t < ST; t++) { acc[t][0] = 0; acc[t][1] = 0; }
-            for (int s = 0; s < wi.nseg; s++) {
-                const double* src = A.partials + (static_cast<size_t>(wi.slot) + s) * (ST * 64);
+            for (int s = 0; s < wm.nseg; s++) {
+                const double* src = A.partials + (static_cast<size_t>(wm.slot) + s) * (ST * 64);
 #pragma unroll
                 for (int t = 0; t < ST; t++) {
                     const double2 v = __ldcg(reinterpret_cast<const double2*>(src + (t * 32 + lane) * 2));
@@ -329,11 +323,19 @@ k_gram(const GramArgs A) {
             continue;
         }
         advance();   // the next WorkItem lands while this owner is being solved
-        if (A.debug_skip_solve & 1) {
-            if (acc[0][0] == 1.2345e300) A.x[0] = acc[ST - 1][1];   // keep the accumulation alive
-            continue;
+        // park the tiles in the slot (over the ring: every lane's copies have landed and been read)
+        __syncwarp();
+        double* const slot = wsm + 2 * lane;
+        const Tiles<64> parked(slot);
+#pragma unroll
+        for (int t = 0; t < ST; t++) parked.st(t, acc[t][0], acc[t][1]);
+        // the next owner's first id batches: in flight during this owner's solve
+        if (w < A.n_work) {
+            first_batches(wi_next);
+            ids_ready = true;
         }
-        gram_solve<M8, GRAM_SOLVE_VARIANT>(acc, n, A.x + static_cast<size_t>(wi.owner) * n,
+        if (A.debug_skip_solve & 1) continue;   // measurement only: the accumulation alone
+        gram_solve_tiles<M8, GRAM_SOLVE_VARIANT, 64>(slot, n, A.x + static_cast<size_t>(wi.owner) * n,
                        A.sse_out ? A.sse_out + wi.owner : nullptr, lane, A,
                        static_cast<size_t>(wi.owner) * n);
     }
@@ -828,19 +830,22 @@ void build_side_lists(Side& sd, const int* d_ptr, int owners, int nnz, int rank,
 template <int M8, bool USER, int EPI>
 void launch_gram(const GramArgs& a, int sms, cudaStream_t s) {
     auto kern = k_gram<M8, USER, EPI>;
-    constexpr int W = gram_warps<USER>();
+    constexpr int W = GRAM_WARPS;
+    constexpr int smem = W * gram_warp_doubles<M8, USER, EPI>() * static_cast<int>(sizeof(double));
+    // per launch: the attribute belongs to the current device
+    MRB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     // one process drives one GPU model; the value is idempotent, so a benign race is excluded by
     // making the cache atomic
     static std::atomic<int> cached{0};
     int per_sm = cached.load(std::memory_order_relaxed);
     if (per_sm == 0) {
-        MRB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, W * 32, 0));
+        MRB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, W * 32, smem));
         cached.store(per_sm, std::memory_order_relaxed);
     }
     MRB_REQUIRE(per_sm >= 1, "gram kernel does not fit on an SM");
     // persistent CTAs: one wave that fills every SM, work items handed out dynamically
     const int grid = std::min(sms * per_sm, ceil_div(a.n_work, W));
-    kern<<<grid > 0 ? grid : 1, W * 32, 0, s>>>(a); MRB_LAUNCHED(1);
+    kern<<<grid > 0 ? grid : 1, W * 32, smem, s>>>(a); MRB_LAUNCHED(1);
     MRB_CUDA(cudaGetLastError());
 }
 

@@ -79,6 +79,29 @@ MRB_DEVICE_INLINE double fast_rsqrt(double d) {
     return fma(fma(e, 0.375, 0.5), y * e, y);
 }
 
+// A lane's fragment tiles, TS doubles apart: tile t is the pair (t * TS, t * TS + 1).  On the GPU
+// they are in shared memory and every access is an explicit ld / st.shared, so that the compiler
+// neither forwards parked values back into registers nor reorders the accesses among themselves
+// (they are all volatile); on the emulated warp they are an ordinary array.
+template <int TS>
+struct Tiles {
+#ifdef MRB_HOST_EMU
+    double* p;
+    explicit Tiles(double* t) : p(t) {}
+    void ld(int t, double& a, double& b) const { a = p[t * TS]; b = p[t * TS + 1]; }
+    void st(int t, double a, double b) const { p[t * TS] = a; p[t * TS + 1] = b; }
+#else
+    unsigned s;
+    __device__ explicit Tiles(double* t) : s(static_cast<unsigned>(__cvta_generic_to_shared(t))) {}
+    __device__ __forceinline__ void ld(int t, double& a, double& b) const {
+        asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(a), "=d"(b) : "r"(s + t * TS * 8));
+    }
+    __device__ __forceinline__ void st(int t, double a, double b) const {
+        asm volatile("st.shared.v2.f64 [%0], {%1, %2};" ::"r"(s + t * TS * 8), "d"(a), "d"(b));
+    }
+#endif
+};
+
 MRB_DEVICE_INLINE double xor_sum_p(double v) {   // sum over the 8 lanes sharing q
     v += __shfl_xor_sync(0xffffffffu, v, 4);
     v += __shfl_xor_sync(0xffffffffu, v, 8);
@@ -92,17 +115,19 @@ MRB_DEVICE_INLINE double xor_sum_q(double v) {   // sum over the 4 lanes sharing
 }
 
 // ------------------------------------------------------------------------------------------
-// K2b: register-resident blocked Cholesky on the mma accumulator fragments.
+// K2b: blocked Cholesky on the mma accumulator fragments.
 //
 // The augmented matrix [G g; g^T s] (order n+1 <= 8*M8) sits in the lower-triangular 8x8 tiles
-// acc[TI(ti,tj)]; lane (p = lane>>2, q = lane&3) holds elements (row p, cols 2q, 2q+1) of every
-// tile.  Right-looking by tile column tk:
+// in fragment order: tile t of lane (p = lane>>2, q = lane&3) is the pair tl[t * TS], tl[t * TS + 1]
+// = elements (row p, cols 2q, 2q+1).  k_gram parks the tiles in a per-warp shared-memory slot
+// (TS = 64, tl = slot + 2 lane), so that only the tiles a step works on occupy registers.
+// Right-looking by tile column tk:
 //   1. the 8 pivot columns of tile column tk are eliminated one by one with warp shuffles
 //      (diagonal tile and the panel tiles below it together);
 //   2. the trailing tiles get  T(ti,tj) -= L(ti,tk) L(tj,tk)^T  on the tensor cores (2 DMMA per
 //      tile; the C-fragment -> A/B-fragment conversion is two shuffles per 8x4 chunk).
 // Row n of the factor is y = L^-1 g', so only the back substitution L^T delta = y remains; it is
-// done on the fragments as well.  No shared memory is used.
+// done on the fragments as well.
 // The system solved is the CORRECTION form  G delta = g - G x0,  x = x0 + delta: an unknown whose
 // pivot as COMPUTED falls below 1e-12 of the original diagonal gets delta = 0 and keeps its
 // previous value (as under the reference's warm-started CG); the others are solved consistently
@@ -128,10 +153,17 @@ MRB_DEVICE_INLINE double xor_sum_q(double v) {   // sum over the 4 lanes sharing
 //  did not help either, 5.97 ms.)
 // (A block-of-four pivot variant was measured and rejected: 7.25 vs 6.63 ms on the user side of
 //  C3, profiles/ab_b4_r02.log.)
-template <int M8, int VARIANT = 0>
-MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
-                                           double* __restrict__ xo, double* __restrict__ sse_slot,
-                                           int lane, const GramArgs& A, size_t row_offset) {
+template <int M8, int VARIANT, int TS>
+MRB_DEVICE_INLINE void gram_solve_tiles(double* tl, int n, double* __restrict__ xo,
+                                        double* __restrict__ sse_slot, int lane, const GramArgs& A,
+                                        size_t row_offset) {
+#ifndef MRB_HOST_EMU
+    // an opaque copy of the lane index: the many lane-derived constants of the solve are formed
+    // per owner instead of being hoisted out of k_gram's owner loop and held live (in registers)
+    // across the accumulation
+    asm volatile("mov.b32 %0, %0;" : "+r"(lane));
+#endif
+    const Tiles<TS> T(tl);
     constexpr int TN = M8 - 1;            // tile row/column holding index n (the rhs)
     const int p = lane >> 2, q = lane & 3;
     const int pr = n & 7;
@@ -158,9 +190,11 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
         for (int ti = 0; ti < M8; ti++)
 #pragma unroll
             for (int tj = 0; tj <= ti; tj++) {
-                colsum[tj][0] += acc[TI(ti, tj)][0] * xp[ti];
-                colsum[tj][1] += acc[TI(ti, tj)][1] * xp[ti];
-                if (ti != tj) rowsum[ti] += acc[TI(ti, tj)][0] * xq[tj][0] + acc[TI(ti, tj)][1] * xq[tj][1];
+                double a0, a1;
+                T.ld(TI(ti, tj), a0, a1);
+                colsum[tj][0] += a0 * xp[ti];
+                colsum[tj][1] += a1 * xp[ti];
+                if (ti != tj) rowsum[ti] += a0 * xq[tj][0] + a1 * xq[tj][1];
             }
 #pragma unroll
         for (int t = 0; t < M8; t++) {
@@ -176,24 +210,34 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
     }
     // ---- rhs' = g - G x0 on the augmented row; x0.(g + g') for the residual bookkeeping
     double gdot = 0;
+    if (p == pr) {
 #pragma unroll
-    for (int t = 0; t < M8; t++)
+        for (int t = 0; t < M8; t++) {
+            double g[2];
+            T.ld(TI(TN, t), g[0], g[1]);
 #pragma unroll
-        for (int s = 0; s < 2; s++) {
-            const int c = 8 * t + 2 * q + s;
-            if (p == pr && c < n) {
-                const double g0 = acc[TI(TN, t)][s];
-                const double g1 = g0 - vy[t][s];
-                acc[TI(TN, t)][s] = g1;
-                gdot += xq[t][s] * (g0 + g1);
+            for (int s = 0; s < 2; s++) {
+                const int c = 8 * t + 2 * q + s;
+                if (c < n) {
+                    const double g0 = g[s];
+                    const double g1 = g0 - vy[t][s];
+                    g[s] = g1;
+                    gdot += xq[t][s] * (g0 + g1);
+                }
             }
+            T.st(TI(TN, t), g[0], g[1]);
         }
+    }
     gdot = xor_sum_q(gdot);   // valid on lanes with p == pr
 
     // ---- pivot thresholds from the original diagonal: lane (p, p>>1) holds column 8t+p's
     double thr[M8];
 #pragma unroll
-    for (int t = 0; t < M8; t++) thr[t] = 1e-12 * ((p & 1) ? acc[TI(t, t)][1] : acc[TI(t, t)][0]);
+    for (int t = 0; t < M8; t++) {
+        double d0, d1;
+        T.ld(TI(t, t), d0, d1);
+        thr[t] = 1e-12 * ((p & 1) ? d1 : d0);
+    }
 
     double invd[M8];   // lane (p, *) : 1/L[j][j] for j = 8t+p (0 for a skipped pivot)
 #pragma unroll
@@ -215,10 +259,14 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
         // control flow around a shuffle) and keeps the pivot columns UNSCALED inside a tile column:
         //   X[p][c2] -= X[p][c] * (D[c2][c] / d_c)      for the 8 pivots c of the tile column,
         // then one scaling of the finished panel by 1/sqrt(d_c) per column.  Per pivot and tile that
-        // is one shuffle and two DFMAs.
+        // is one shuffle and two DFMAs.  The diagonal tile is held in registers for its tile column;
+        // every other tile is read when its column or its trailing update needs it and written back.
+        double dnext[2];   // the diagonal tile of the next column, straight from the trailing update
+        T.ld(0, dnext[0], dnext[1]);
     #pragma unroll
         for (int tk = 0; tk < M8; tk++) {
             const int D = TI(tk, tk);
+            double d[2] = {dnext[0], dnext[1]};
             // the 8 pivot columns, rolled in pairs (cp = c >> 1 at run time, slot j = c & 1 static):
             // 4x less code than a full unroll -- the epilogue was instruction-cache bound (a full
             // unroll measured 9.78 vs 9.70 ms per C3 sweep, profiles/ab_unroll_r02.log)
@@ -231,7 +279,7 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
                     if (tk < M8 - 1 || c < pr) {
                         // the owner lane (p = c, q = cp) holds d = D[c][c] in slot j and its threshold
                         // in thr[tk]; every lane runs the reciprocal square root on its own value
-                        const double dv = acc[D][j];
+                        const double dv = d[j];
                         const bool ok = dv > thr[tk] && thr[tk] > 1e-290;   // false for NaN
                         const double r = shfl_double(ok ? fast_rsqrt(dv) : 0.0, c * 4 + cp);
                         if (p == c) invd[tk] = r;
@@ -242,12 +290,18 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
                             const double m1 = shfl_double(dv, (2 * q + 1) * 4 + cp);
                             const double f0 = q > cp ? m0 * inv_d : 0.0;
                             const double f1 = (j == 0 ? q >= cp : q > cp) ? m1 * inv_d : 0.0;
+                            {
+                                const double xrc = shfl_double(d[j], p * 4 + cp);   // X[p][c]
+                                d[0] = fma(-xrc, f0, d[0]);
+                                d[1] = fma(-xrc, f1, d[1]);
+                            }
     #pragma unroll
-                            for (int ti = tk; ti < (WPANEL ? tk + 1 : M8); ti++) {
+                            for (int ti = tk + 1; ti < (WPANEL ? tk + 1 : M8); ti++) {
                                 const int X = TI(ti, tk);
-                                const double xrc = shfl_double(acc[X][j], p * 4 + cp);   // X[p][c]
-                                acc[X][0] = fma(-xrc, f0, acc[X][0]);
-                                acc[X][1] = fma(-xrc, f1, acc[X][1]);
+                                double x0, x1;
+                                T.ld(X, x0, x1);
+                                const double xrc = shfl_double(j ? x1 : x0, p * 4 + cp);
+                                T.st(X, fma(-xrc, f0, x0), fma(-xrc, f1, x1));
                             }
                             if (WSUB) {
                                 const double wrc = shfl_double(Wt[WSUB ? tk : 0][j], p * 4 + cp);
@@ -258,21 +312,27 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
                     }
                 }
             }
-            if (tk == M8 - 1) corner = (pr & 1) ? acc[D][1] : acc[D][0];   // valid on lane (pr, pr>>1)
+            if (tk == M8 - 1) corner = (pr & 1) ? d[1] : d[0];   // valid on lane (pr, pr>>1)
             {
                 // L = X diag(1/sqrt(d)); skipped pivots and the non-pivot columns become 0
                 const double r0 = shfl_double(invd[tk], (2 * q) * 4);
                 const double r1 = shfl_double(invd[tk], (2 * q + 1) * 4);
+                d[0] *= r0;
+                d[1] *= r1;
+                T.st(D, d[0], d[1]);
     #pragma unroll
-                for (int ti = tk; ti < (WPANEL ? tk + 1 : M8); ti++) {
-                    acc[TI(ti, tk)][0] *= r0;
-                    acc[TI(ti, tk)][1] *= r1;
+                for (int ti = tk + 1; ti < (WPANEL ? tk + 1 : M8); ti++) {
+                    double x0, x1;
+                    T.ld(TI(ti, tk), x0, x1);
+                    T.st(TI(ti, tk), x0 * r0, x1 * r1);
                 }
                 if (WSUB) {
                     Wt[WSUB ? tk : 0][0] *= r0;
                     Wt[WSUB ? tk : 0][1] *= r1;
                 }
             }
+            // the finished panel L(ti, tk), ti > tk, in registers for the trailing update
+            double pan[M8][2];
             if (WPANEL && tk < M8 - 1) {
                 // W^T as a C fragment: lane (p, q) slot s holds W[2q + s][p] -- which is element
                 // (k = q, column p) of the B operand over the rows {2q + s} of W
@@ -288,12 +348,18 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
     #pragma unroll
                 for (int ti = tk + 1; ti < M8; ti++) {
                     const int X = TI(ti, tk);
+                    double x0, x1;
+                    T.ld(X, x0, x1);
                     double c0 = 0.0, c1 = 0.0;
-                    dmma884(c0, c1, acc[X][0], wT[0]);
-                    dmma884(c0, c1, acc[X][1], wT[1]);
-                    acc[X][0] = c0;
-                    acc[X][1] = c1;
+                    dmma884(c0, c1, x0, wT[0]);
+                    dmma884(c0, c1, x1, wT[1]);
+                    T.st(X, c0, c1);
+                    pan[ti][0] = c0;
+                    pan[ti][1] = c1;
                 }
+            } else if (tk < M8 - 1) {
+    #pragma unroll
+                for (int ti = tk + 1; ti < M8; ti++) T.ld(TI(ti, tk), pan[ti][0], pan[ti][1]);
             }
             if (tk < M8 - 1) {
                 // trailing update on the tensor cores: T(ti,tj) -= L(ti,tk) L(tj,tk)^T
@@ -306,8 +372,8 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
     #pragma unroll
                     for (int h = 0; h < 2; h++) {
                         const int src = p * 4 + 2 * h + (q >> 1);
-                        const double v0 = shfl_double(acc[TI(ti, tk)][0], src);
-                        const double v1 = shfl_double(acc[TI(ti, tk)][1], src);
+                        const double v0 = shfl_double(pan[ti][0], src);
+                        const double v1 = shfl_double(pan[ti][1], src);
                         ax[ti][h] = (q & 1) ? v1 : v0;   // L(ti,tk)[p][4h+q]
                     }
     #else
@@ -316,19 +382,22 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
                 // Lane (p, q) holds L[p][2q + h] in slot h of the C fragment, which is exactly
                 // element (row p, k = q) of an A fragment and (k = q, column p) of a B fragment
                 // over the columns {2q + h}: no data movement at all.
-                double ax[M8][2];
-    #pragma unroll
-                for (int ti = tk + 1; ti < M8; ti++) {
-                    ax[ti][0] = acc[TI(ti, tk)][0];
-                    ax[ti][1] = acc[TI(ti, tk)][1];
-                }
+                double (&ax)[M8][2] = pan;
     #endif
     #pragma unroll
                 for (int ti = tk + 1; ti < M8; ti++)
     #pragma unroll
                     for (int tj = tk + 1; tj <= ti; tj++) {
-                        dmma884(acc[TI(ti, tj)][0], acc[TI(ti, tj)][1], -ax[ti][0], ax[tj][0]);
-                        dmma884(acc[TI(ti, tj)][0], acc[TI(ti, tj)][1], -ax[ti][1], ax[tj][1]);
+                        double t0, t1;
+                        T.ld(TI(ti, tj), t0, t1);
+                        dmma884(t0, t1, -ax[ti][0], ax[tj][0]);
+                        dmma884(t0, t1, -ax[ti][1], ax[tj][1]);
+                        if (ti == tk + 1) {   // the next diagonal tile: stays in registers
+                            dnext[0] = t0;
+                            dnext[1] = t1;
+                        } else {
+                            T.st(TI(ti, tj), t0, t1);
+                        }
                     }
             }
         }
@@ -350,18 +419,21 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
         // last tile) make the corresponding delta exactly 0.
 #pragma unroll
         for (int tj = M8 - 1; tj >= 0; tj--) {
-            double yv[2];
+            double yv[2], yr[2];
+            T.ld(TI(TN, tj), yr[0], yr[1]);
 #pragma unroll
             for (int s = 0; s < 2; s++) {
-                yv[s] = shfl_double(acc[TI(TN, tj)][s], pr * 4 + q);
+                yv[s] = shfl_double(yr[s], pr * 4 + q);
                 if (tj < M8 - 1) yv[s] -= xor_sum_p(part[tj][s]);
             }
             const int wt = WSUB ? tj : 0;
             const double dp = xor_sum_q(fma(Wt[wt][0], yv[0], Wt[wt][1] * yv[1]));   // delta[8 tj + p]
 #pragma unroll
             for (int t2 = 0; t2 < tj; t2++) {
-                part[t2][0] = fma(acc[TI(tj, t2)][0], dp, part[t2][0]);
-                part[t2][1] = fma(acc[TI(tj, t2)][1], dp, part[t2][1]);
+                double l0, l1;
+                T.ld(TI(tj, t2), l0, l1);
+                part[t2][0] = fma(l0, dp, part[t2][0]);
+                part[t2][1] = fma(l1, dp, part[t2][1]);
             }
             xq[tj][0] += shfl_double(dp, (2 * q) * 4);
             xq[tj][1] += shfl_double(dp, (2 * q + 1) * 4);
@@ -370,13 +442,16 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
 #pragma unroll
     for (int tj = M8 - 1; tj >= 0; tj--) {
         const int D = TI(tj, tj);
-        double yv[2], rq[2], dlt[2] = {0.0, 0.0};
+        double yv[2], rq[2], dlt[2] = {0.0, 0.0}, yr[2];
+        T.ld(TI(TN, tj), yr[0], yr[1]);
 #pragma unroll
         for (int s = 0; s < 2; s++) {
-            yv[s] = shfl_double(acc[TI(TN, tj)][s], pr * 4 + q);
+            yv[s] = shfl_double(yr[s], pr * 4 + q);
             if (tj < M8 - 1) yv[s] -= xor_sum_p(part[tj][s]);
             rq[s] = shfl_double(invd[tj], (2 * q + s) * 4);
         }
+        double dd[2];
+        T.ld(D, dd[0], dd[1]);
 #pragma unroll 1
         for (int cp = 3; cp >= 0; cp--) {
 #pragma unroll
@@ -386,8 +461,8 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
                     const double dc = shfl_double(yv[j] * rq[j], cp);   // delta[8 tj + c]
                     if (q == cp) dlt[j] = dc;
                     if (c > 0) {
-                        const double l0 = shfl_double(acc[D][0], c * 4 + q);   // L[c][2q]
-                        const double l1 = shfl_double(acc[D][1], c * 4 + q);   // L[c][2q+1]
+                        const double l0 = shfl_double(dd[0], c * 4 + q);   // L[c][2q]
+                        const double l1 = shfl_double(dd[1], c * 4 + q);   // L[c][2q+1]
                         const double d0 = (j == 0 ? q < cp : q <= cp) ? dc : 0.0;
                         const double d1 = q < cp ? dc : 0.0;
                         yv[0] = fma(-l0, d0, yv[0]);
@@ -402,8 +477,10 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
             const double dp = (p & 1) ? v1 : v0;   // delta[8 tj + p] (0 for rows >= n)
 #pragma unroll
             for (int t2 = 0; t2 < tj; t2++) {
-                part[t2][0] = fma(acc[TI(tj, t2)][0], dp, part[t2][0]);
-                part[t2][1] = fma(acc[TI(tj, t2)][1], dp, part[t2][1]);
+                double l0, l1;
+                T.ld(TI(tj, t2), l0, l1);
+                part[t2][0] = fma(l0, dp, part[t2][0]);
+                part[t2][1] = fma(l1, dp, part[t2][1]);
             }
         }
         xq[tj][0] += dlt[0];
@@ -432,6 +509,14 @@ MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
             for (int j = 0; j < A.n_peers; j++) A.x_peers[j][row_offset + c] = lin[h];
         }
     }
+}
+
+// The same on a lane's own register array acc[TI(ti,tj)][h] (the emulated warp of tests/emu).
+template <int M8, int VARIANT = 0>
+MRB_DEVICE_INLINE void gram_solve(double (&acc)[M8 * (M8 + 1) / 2][2], int n,
+                                  double* __restrict__ xo, double* __restrict__ sse_slot,
+                                  int lane, const GramArgs& A, size_t row_offset) {
+    gram_solve_tiles<M8, VARIANT, 2>(&acc[0][0], n, xo, sse_slot, lane, A, row_offset);
 }
 
 }  // namespace
