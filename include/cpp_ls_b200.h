@@ -225,6 +225,58 @@ MRB_API int mrb_als_shard_sse(mrb_als_problem* p, void* stream, double* out);
 MRB_API int mrb_als_stream_sync(mrb_als_problem* p, void* stream);
 /* CUDA-event time (ms) summed over the half-sweep launches since the last call. */
 MRB_API int mrb_als_collect_gram_ms(mrb_als_problem* p, float* out);
+
+/* ---- algorithm 3 (Gram block-CG) over the peer group -----------------------------------------
+ * The reference's CG (global alpha and beta, its stopping rule, inner (0.01, 200)) on per-row
+ * Gram blocks, with the work split so that the factors, the CG iteration counts and final_rr are
+ * bit-identical to one-GPU algorithm 3 for every world size.  Row work (Gram store, block matvec)
+ * is done by the rank a row is dealt to, which keeps only its own rows' blocks (about 1/world of
+ * the Gram memory).  Vector work is done by the rank owning the element's 256-element chunk: rank
+ * r owns chunks [vb r / world, vb (r+1) / world) of the vb = ceil(len / 256) chunks of a side.
+ * Outputs move by peer stores into one exchange block per rank; the scalar steps run on every rank.
+ *
+ * Setup, once, after mrb_als_set_shard or mrb_als_open_peers_all: mrb_als_cg_prepare on every
+ * rank; then either mrb_als_cg_exchange_handle, exchange the 64-byte handles, mrb_als_cg_open_peers
+ * and a peer barrier (no rank may begin before every block is zeroed), or -- ranks emulated in one
+ * process -- mrb_als_cg_exchange_block and mrb_als_cg_set_peer_pointers.
+ *
+ * One half-sweep (B = mrb_als_peer_barrier, enqueued by the caller on the same stream; every rank
+ * issues the same sequence):
+ *   mrb_als_cg_begin | B | phase RESIDUAL | B | phase INIT ; mrb_als_cg_state
+ *   while not done: 4 x [ phase MATVEC | B | phase XR | B | phase P | B ] ; mrb_als_cg_state
+ *   mrb_als_cg_finish | B
+ * The iterations of a batch are guarded on the device: after the stop they do nothing, but their
+ * barriers are still enqueued, so every rank keeps the same barrier sequence.  None of these calls
+ * enqueues a barrier; all of them enqueue on `stream` without synchronising except
+ * mrb_als_cg_state, which synchronises `stream` and reads this rank's copy of the CG state (every
+ * rank's copy is the same). */
+#define MRB_CG_PHASE_RESIDUAL 0   /* chunk range: r = Ap - g, p = -r, r.r partials */
+#define MRB_CG_PHASE_INIT 1       /* local: rr and the stopping state from the partials */
+#define MRB_CG_PHASE_MATVEC 2     /* owned rows: Ap = G p, per-owner dots */
+#define MRB_CG_PHASE_XR 3         /* alpha; chunk range: x += alpha p, r += alpha Ap, partials */
+#define MRB_CG_PHASE_P 4          /* beta and the stopping rule; chunk range: p = beta p - r */
+/* Host-only: out[o] = the rank owner o is dealt to, -1 for an owner without ratings. */
+MRB_API int mrb_owner_ranks(const int* ptr, int owners, int world, int* out);
+/* Allocates the compact Gram blocks of this rank's rows, the exchange block (zeroed) and the
+ * owner -> rank maps; synchronises.  Idempotent. */
+MRB_API int mrb_als_cg_prepare(mrb_als_problem* p);
+/* 64 bytes: IPC handle of the exchange block (pinned like the blocks of mrb_als_ipc_handles_all). */
+MRB_API int mrb_als_cg_exchange_handle(mrb_als_problem* p, unsigned char* handle64);
+/* handles_by_rank: world x 64 bytes, world as given to mrb_als_open_peers_all. */
+MRB_API int mrb_als_cg_open_peers(mrb_als_problem* p, const unsigned char* handles_by_rank, int world);
+MRB_API int mrb_als_cg_exchange_block(mrb_als_problem* p, void** d_block);
+/* Every rank's exchange block as device pointers valid in this process; entry `rank` is ignored. */
+MRB_API int mrb_als_cg_set_peer_pointers(mrb_als_problem* p, void* const* d_blocks, int world);
+/* Gram blocks of this rank's rows of one side (user_side != 0: users) and the initial matvec on
+ * the factors; after the barrier that follows, the Ap and g of every chunk have arrived. */
+MRB_API int mrb_als_cg_begin(mrb_als_problem* p, int user_side, void* stream);
+MRB_API int mrb_als_cg_phase(mrb_als_problem* p, int phase, void* stream);
+/* done (0: iterate on; 1: slow decrease; 2: max iterations or rr < 1e-6), iterations, final_rr. */
+MRB_API int mrb_als_cg_state(mrb_als_problem* p, void* stream, int* done, int* iterations,
+                             double* final_rr);
+/* This rank's chunk range of the solved side's factors into every other replica; after the
+ * barrier that follows, every replica holds the complete factors. */
+MRB_API int mrb_als_cg_finish(mrb_als_problem* p, void* stream);
 /* Kernels launched by this library in this process so far. */
 MRB_API long long mrb_kernel_launches(void);
 

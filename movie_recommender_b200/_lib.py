@@ -127,6 +127,19 @@ def _declare(dll):
     dll.mrb_als_stream_sync.argtypes = [c_void_p, c_void_p]
     dll.mrb_als_shard_sse.restype = c_int
     dll.mrb_als_shard_sse.argtypes = [c_void_p, c_void_p, _D]
+    dll.mrb_owner_ranks.restype = c_int
+    dll.mrb_owner_ranks.argtypes = [_I, c_int, c_int, _I]
+    for name, args in (("mrb_als_cg_prepare", [c_void_p]),
+                       ("mrb_als_cg_exchange_handle", [c_void_p, _B]),
+                       ("mrb_als_cg_open_peers", [c_void_p, _B, c_int]),
+                       ("mrb_als_cg_exchange_block", [c_void_p, ctypes.POINTER(c_void_p)]),
+                       ("mrb_als_cg_set_peer_pointers", [c_void_p, ctypes.POINTER(c_void_p), c_int]),
+                       ("mrb_als_cg_begin", [c_void_p, c_int, c_void_p]),
+                       ("mrb_als_cg_phase", [c_void_p, c_int, c_void_p]),
+                       ("mrb_als_cg_state", [c_void_p, c_void_p, _I, _I, _D]),
+                       ("mrb_als_cg_finish", [c_void_p, c_void_p])):
+        getattr(dll, name).restype = c_int
+        getattr(dll, name).argtypes = args
     dll.mrb_als_collect_gram_ms.restype = c_int
     dll.mrb_als_collect_gram_ms.argtypes = [c_void_p, ctypes.POINTER(ctypes.c_float)]
     dll.mrb_cosine_topk.restype = c_int

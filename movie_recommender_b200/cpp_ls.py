@@ -332,6 +332,45 @@ class AlsProblem:
                                           ctypes.cast(ctypes.byref(out), _lib._D)))
         return out.value
 
+    # ---- algorithm 3 over the peer group, phase by phase (sharded.gram_cg_half_sweep drives it)
+    def cg_prepare(self):
+        _lib.check(_dll.mrb_als_cg_prepare(self._h))
+
+    def cg_exchange_handle(self):
+        h = (ctypes.c_ubyte * 64)()
+        _lib.check(_dll.mrb_als_cg_exchange_handle(self._h, h))
+        return bytes(h)
+
+    def cg_open_peers(self, handles_by_rank):
+        world = len(handles_by_rank)
+        buf = (ctypes.c_ubyte * (64 * world)).from_buffer_copy(b"".join(handles_by_rank))
+        _lib.check(_dll.mrb_als_cg_open_peers(self._h, buf, world))
+
+    def cg_exchange_block(self):
+        b = ctypes.c_void_p()
+        _lib.check(_dll.mrb_als_cg_exchange_block(self._h, ctypes.byref(b)))
+        return b.value
+
+    def cg_set_peer_pointers(self, blocks):
+        arr = (ctypes.c_void_p * len(blocks))(*blocks)
+        _lib.check(_dll.mrb_als_cg_set_peer_pointers(self._h, arr, len(blocks)))
+
+    def cg_begin(self, user_side, stream):
+        _lib.check(_dll.mrb_als_cg_begin(self._h, 1 if user_side else 0, ctypes.c_void_p(stream)))
+
+    def cg_phase(self, phase, stream):
+        _lib.check(_dll.mrb_als_cg_phase(self._h, phase, ctypes.c_void_p(stream)))
+
+    def cg_state(self, stream):
+        """(done, iterations, final_rr) of the running half-sweep; synchronises ``stream``."""
+        done, it, rr = ctypes.c_int(0), ctypes.c_int(0), ctypes.c_double(0)
+        _lib.check(_dll.mrb_als_cg_state(self._h, ctypes.c_void_p(stream), ctypes.byref(done),
+                                         ctypes.byref(it), ctypes.cast(ctypes.byref(rr), _lib._D)))
+        return done.value, it.value, rr.value
+
+    def cg_finish(self, stream):
+        _lib.check(_dll.mrb_als_cg_finish(self._h, ctypes.c_void_p(stream)))
+
     def collect_gram_ms(self):
         out = ctypes.c_float(0)
         _lib.check(_dll.mrb_als_collect_gram_ms(self._h, ctypes.byref(out)))
@@ -346,6 +385,14 @@ def dealt_owners(ptr, rank, world):
     out = numpy.zeros(owners // world + 1, dtype=numpy.int32)
     m = _lib.check(_dll.mrb_dealt_owners(_lib.ip(ptr), owners, world, rank, _lib.ip(out)))
     return out[:m]
+
+
+def owner_ranks(ptr, world):
+    """Host only: the rank each row is dealt to (-1 for a row without ratings)."""
+    ptr = numpy.ascontiguousarray(ptr, dtype=numpy.int32)
+    out = numpy.zeros(max(len(ptr) - 1, 1), dtype=numpy.int32)
+    _lib.check(_dll.mrb_owner_ranks(_lib.ip(ptr), len(ptr) - 1, world, _lib.ip(out)))
+    return out[:len(ptr) - 1]
 
 
 def kernel_launches():

@@ -22,6 +22,13 @@ enum AlsAlgorithm : int {
     ALS_GRAM_CHOLESKY = 4  // per-row normal equations solved exactly (in-shared-memory Cholesky)
 };
 
+using CgState = FaithfulCG::State;
+// phases of one sharded CG half-sweep (values of MRB_CG_PHASE_* in cpp_ls_b200.h)
+enum CgPhase : int { CG_PHASE_RESIDUAL = 0, CG_PHASE_INIT = 1, CG_PHASE_MATVEC = 2, CG_PHASE_XR = 3,
+                     CG_PHASE_P = 4 };
+// Host inverse of the dealt partition: out[o] = rank owner o is dealt to, -1 without ratings.
+void owner_ranks_host(const int* ptr, int owners, int world, int* out);
+
 struct AlsRunInfo {
     int sweeps_returned = 0;   // the reference's return value (sweep counter at exit)
     int sweeps_run = 0;        // number of (user, item) half-sweep pairs executed
@@ -99,6 +106,17 @@ public:
     double shard_sse(cudaStream_t stream);
     float collect_gram_ms();   // CUDA-event time of the half_sweep launches since the last call
 
+    // ---- algorithm 3 (Gram block-CG) with the rows dealt over the ranks, driven phase by phase
+    // (the phase order and its barriers: als_gram.cu, "algorithm 3 with rows dealt over several
+    // GPUs").  Factors, iteration counts and final_rr equal one-GPU algorithm 3 bit for bit.
+    void cg_prepare();                       // compact Gram blocks, exchange block, owner -> rank maps
+    double* cg_exchange_block();             // this rank's exchange block (to export or share)
+    void set_cg_peers(const std::vector<double*>& blocks);   // index = rank (own entry ignored)
+    void cg_begin(bool user_side, cudaStream_t stream);      // Gram store + initial matvec (row)
+    void cg_phase(int phase, cudaStream_t stream);           // CG_PHASE_*
+    CgState cg_state(cudaStream_t stream);                   // synchronises stream
+    void cg_finish(cudaStream_t stream);     // this rank's chunk range of x into every replica
+
     int nnz() const { return nnz_; }
     int k() const { return k_; }
     int num_users() const { return nu_; }
@@ -118,7 +136,8 @@ private:
     void ensure_gram();
     void wait_ratings();   // s_ waits for the ratings upload (second stream)
     void wait_factors();   // s_ waits for a pending set_factors_async
-    void launch_half(bool user_side, cudaStream_t stream, int epilogue);
+    void launch_half(bool user_side, cudaStream_t stream, int epilogue, bool compact = false);
+    void cg_matvec(const double* v, const double* g_c, const CgState* guard, cudaStream_t stream);
     void destroy_handles();
     void check_ids();
 

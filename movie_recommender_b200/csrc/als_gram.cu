@@ -302,9 +302,11 @@ k_gram(const GramArgs A) {
         }
 
         if (EPI == EPI_STORE) {
-            // algorithm 3: G (row-major n x n, both triangles) and g to HBM
-            double* Go = A.G_out + static_cast<size_t>(wi.owner) * n * n;
-            double* go = A.g_out + static_cast<size_t>(wi.owner) * n;
+            // algorithm 3: G (row-major n x n, both triangles) and g to HBM, indexed by owner
+            // (one GPU) or by the owner's compact slot (rows dealt over several GPUs)
+            const size_t blk = static_cast<size_t>(A.store_by_slot ? wi.pad : wi.owner);
+            double* Go = A.G_out + blk * n * n;
+            double* go = A.g_out + blk * n;
 #pragma unroll
             for (int ti = 0; ti < M8; ti++)
 #pragma unroll
@@ -581,7 +583,7 @@ __global__ void k_gather_grouped(const int* __restrict__ idx, const int* __restr
 
 // Host mirror of the dealt partition (k_lpt_keys + stable_group_by + k_deal_order): the owners
 // rank r receives, in its processing order.  Used by the CPU tests of the N > 1 host logic.
-int dealt_owners_host(const int* ptr, int owners, int world, int rank, int* out) {
+static std::vector<int> lpt_order_host(const int* ptr, int owners) {
     std::vector<int> order(static_cast<size_t>(owners));
     std::iota(order.begin(), order.end(), 0);
     auto key = [&](int o) {
@@ -589,6 +591,11 @@ int dealt_owners_host(const int* ptr, int owners, int world, int rank, int* out)
         return deg >= 65535 ? 0 : 65535 - deg;
     };
     std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return key(a) < key(b); });
+    return order;
+}
+
+int dealt_owners_host(const int* ptr, int owners, int world, int rank, int* out) {
+    const std::vector<int> order = lpt_order_host(ptr, owners);
     const int full = owners / world, rest = owners % world;
     const int m = full + (rank < rest ? 1 : 0);
     for (int t = 0; t < m; t++) {
@@ -596,6 +603,19 @@ int dealt_owners_host(const int* ptr, int owners, int world, int rank, int* out)
         out[t] = order[static_cast<size_t>(t) * world + off];
     }
     return m;
+}
+
+// The inverse of the deal: out[o] = the rank owner o is dealt to, -1 for an owner without ratings
+// (it is in no rank's work list).  Sorted position q = t world + j of block t goes to rank j, or
+// to world-1-j in the odd complete blocks.
+void owner_ranks_host(const int* ptr, int owners, int world, int* out) {
+    const std::vector<int> order = lpt_order_host(ptr, owners);
+    const int full = owners / world;
+    for (int q = 0; q < owners; q++) {
+        const int t = q / world, j = q % world;
+        const int o = order[static_cast<size_t>(q)];
+        out[o] = ptr[o + 1] > ptr[o] ? ((t < full && (t & 1)) ? world - 1 - j : j) : -1;
+    }
 }
 
 namespace {
@@ -736,7 +756,7 @@ __global__ void k_write_work(const int* __restrict__ ptr, int m,
         wi.nseg = nseg;
         wi.slot = nseg > 1 ? slot_at[j] : 0;
         wi.multi = nseg > 1 ? multi_at[j] : -1;
-        wi.pad = 0;
+        wi.pad = nonempty_at[j];
         work[item_at[j] + sg] = wi;
     }
 }
@@ -877,17 +897,19 @@ namespace {
 // dots, then one fixed-order reduction.
 // ------------------------------------------------------------------------------------------
 
+// the replicas a range of factor rows is stored into besides the local one
+struct PeerRows {
+    double* x_peers[8];
+    int n_peers;
+};
+
+// y = G_o v_o for one owner's n x n block (one warp, lanes along the row) and d = v_o . y summed
+// over the warp; the one arithmetic of the one-GPU and the owned-rows matvec
 template <int NPL>   // unknowns per lane: n <= 32 * NPL
-__global__ void __launch_bounds__(256)
-k_block_matvec(const double* __restrict__ G, const double* __restrict__ v, double* __restrict__ out,
-               double* __restrict__ dots, int owners, int n, const CgState* __restrict__ guard) {
-    if (guard && guard->done) return;
-    const int o = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (o >= owners) return;
-    const int lane = threadIdx.x & 31;
-    const double* Go = G + static_cast<size_t>(o) * n * n;
-    const double* vo = v + static_cast<size_t>(o) * n;
-    double vv[NPL], y[NPL];
+__device__ __forceinline__ double block_row_matvec(const double* __restrict__ Go,
+                                                   const double* __restrict__ vo, int n, int lane,
+                                                   double (&y)[NPL]) {
+    double vv[NPL];
 #pragma unroll
     for (int m = 0; m < NPL; m++) {
         vv[m] = lane + 32 * m < n ? vo[lane + 32 * m] : 0.0;
@@ -905,16 +927,72 @@ k_block_matvec(const double* __restrict__ G, const double* __restrict__ v, doubl
                 if (lane + 32 * m < n) y[m] += row[lane + 32 * m] * vj;
         }
     }
-    double* oo = out + static_cast<size_t>(o) * n;
     double d = 0;
 #pragma unroll
-    for (int m = 0; m < NPL; m++) {
-        if (lane + 32 * m < n) oo[lane + 32 * m] = y[m];
-        d += vv[m] * y[m];
-    }
+    for (int m = 0; m < NPL; m++) d += vv[m] * y[m];
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) d += __shfl_xor_sync(0xffffffffu, d, off);
+    return d;
+}
+
+template <int NPL>
+__global__ void __launch_bounds__(256)
+k_block_matvec(const double* __restrict__ G, const double* __restrict__ v, double* __restrict__ out,
+               double* __restrict__ dots, int owners, int n, const CgState* __restrict__ guard) {
+    if (guard && guard->done) return;
+    const int o = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (o >= owners) return;
+    const int lane = threadIdx.x & 31;
+    double y[NPL];
+    const double d = block_row_matvec<NPL>(G + static_cast<size_t>(o) * n * n,
+                                           v + static_cast<size_t>(o) * n, n, lane, y);
+    double* oo = out + static_cast<size_t>(o) * n;
+#pragma unroll
+    for (int m = 0; m < NPL; m++)
+        if (lane + 32 * m < n) oo[lane + 32 * m] = y[m];
     if (lane == 0) dots[o] = d;
+}
+
+// The block matvec over this rank's owned rows (sharded algorithm 3): warp t takes owner
+// owner_order[t] and its compact block G[t]; Ap goes to the rank owning each element's chunk (a
+// row may straddle two ranks' chunk ranges), dots[o] to every rank.  With g_c (the compact g of
+// the Gram store; the initial matvec only) g is routed along with Ap.
+template <int NPL>
+__global__ void __launch_bounds__(256)
+k_block_matvec_owned(const double* __restrict__ G, const double* __restrict__ g_c,
+                     const int* __restrict__ owner_order, int n_owned, const double* __restrict__ v,
+                     const CgRoute route, const CgState* __restrict__ guard) {
+    if (guard && guard->done) return;
+    const int t = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (t >= n_owned) return;
+    const int lane = threadIdx.x & 31;
+    const int n = route.n;
+    const int o = owner_order[t];
+    double y[NPL];
+    const double d = block_row_matvec<NPL>(G + static_cast<size_t>(t) * n * n,
+                                           v + static_cast<size_t>(o) * n, n, lane, y);
+#pragma unroll
+    for (int m = 0; m < NPL; m++) {
+        const int j = lane + 32 * m;
+        if (j >= n) continue;
+        const int e = o * n + j;
+        int q = 0;
+        while (q + 1 < route.world && (e >> 8) >= route.chunk_lo[q + 1]) q++;
+        route.Ap[q][e] = y[m];
+        if (g_c) route.g[q][e] = g_c[static_cast<size_t>(t) * n + j];
+    }
+    if (lane < route.world) route.dots[lane][o] = d;
+}
+
+// x[lo, hi) of this rank's replica into the other replicas (the chunk range a rank updated)
+__global__ void k_store_range(const double* __restrict__ x, long long lo, long long hi,
+                              const PeerRows peers) {
+    const long long i = lo + static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (i >= hi) return;
+    const double v = x[i];
+#pragma unroll
+    for (int q = 0; q < 8; q++)
+        if (q < peers.n_peers) peers.x_peers[q][i] = v;
 }
 
 }  // namespace
@@ -971,6 +1049,36 @@ void set_peer_targets(Args& a, const std::vector<double*>& peers, int rank) {
         if (static_cast<int>(j) != rank && peers[j] != nullptr && a.n_peers < 8)
             a.x_peers[a.n_peers++] = peers[j];
 }
+
+// Offsets (in doubles) of one side's arrays in the exchange block.
+struct CgRegion {
+    int owners = 0, n = 1, len = 0, vb = 1;
+    size_t r = 0, p = 0, Ap = 0, g = 0, dots = 0, partials = 0, state = 0, end = 0;
+};
+
+CgRegion cg_region(int owners, int n, size_t base) {
+    CgRegion c;
+    c.owners = owners;
+    c.n = n;
+    c.len = owners * n;
+    c.vb = ceil_div(c.len > 0 ? c.len : 1, 256);
+    const size_t len = static_cast<size_t>(std::max(c.len, 1));
+    c.r = base;
+    c.p = c.r + len;
+    c.Ap = c.p + len;
+    c.g = c.Ap + len;
+    c.dots = c.g + len;
+    c.partials = c.dots + static_cast<size_t>(std::max(owners, 1));
+    c.state = c.partials + c.vb + 1;   // (the last partial holds the reduced scalar)
+    c.end = c.state + (sizeof(CgState) + sizeof(double) - 1) / sizeof(double);
+    return c;
+}
+
+// Rank r's chunks of a side: the contiguous 1/world share of its vb 256-element chunks.
+inline int cg_chunk_lo(int vb, int r, int world) {
+    return static_cast<int>(static_cast<long long>(vb) * r / world);
+}
+
 }  // namespace
 
 struct AlsProblem::GramState {
@@ -990,6 +1098,15 @@ struct AlsProblem::GramState {
     // algorithm 3 (Gram block-CG): stored blocks and CG vectors, sized for the larger side
     DevBuf<double> G, g, r, p, Ap, dots, cg_partials;
     DevBuf<FaithfulCG::State> cg_state;
+    // algorithm 3 with rows dealt over several GPUs (cg_prepare): the Gram blocks of this rank's
+    // owners by compact slot (position in the side's owner_order), the owner -> rank maps, and the
+    // exchange block -- per side r, p, Ap, g, dots, partials and the CG state, at the same offsets
+    // on every rank, so that a peer's base pointer locates every array
+    DevBuf<double> oG, og, xb;
+    DevBuf<int> user_rank, item_rank;
+    CgRegion cg_user, cg_item;
+    std::vector<double*> xb_peers;   // index = rank
+    bool cg_on_user = true, cg_begun = false;
 };
 
 void AlsProblem::ensure_gram() {
@@ -1044,7 +1161,8 @@ void AlsProblem::ensure_gram() {
 }
 
 // One k_gram launch (algorithm 4) over this rank's rows of one side, timed by a pair of events.
-void AlsProblem::launch_half(bool user_side, cudaStream_t stream, int epilogue) {
+// compact (EPI_STORE only): the blocks of this rank's owners by compact slot (sharded algorithm 3).
+void AlsProblem::launch_half(bool user_side, cudaStream_t stream, int epilogue, bool compact) {
     GramState& g = *gram_;
     Side& sd = user_side ? g.user : g.item;
     if (g.wide_fused && epilogue == EPI_SOLVE) {
@@ -1128,20 +1246,23 @@ void AlsProblem::launch_half(bool user_side, cudaStream_t stream, int epilogue) 
         gram_events_.push_back(e1);
         MRB_CUDA(cudaEventRecord(e0, stream));
         const bool store = epilogue == EPI_STORE;
+        double* const sG = compact ? g.oG.p : g.G.p;
+        double* const sg = compact ? g.og.p : g.g.p;
         if (store) {
-            const size_t owners = user_side ? nu_ : ni_;
-            MRB_CUDA(cudaMemsetAsync(g.G.p, 0, sizeof(double) * owners * n * n, stream));
-            MRB_CUDA(cudaMemsetAsync(g.g.p, 0, sizeof(double) * owners * n, stream));
+            const size_t owners = compact ? sd.n_owner_items : (user_side ? nu_ : ni_);
+            MRB_CUDA(cudaMemsetAsync(sG, 0, sizeof(double) * owners * n * n, stream));
+            MRB_CUDA(cudaMemsetAsync(sg, 0, sizeof(double) * owners * n, stream));
         }
+        // (the store batch is the whole owner_order: the batch position is the compact slot)
         const int batch = store ? sd.n_owner_items : g.wide_batch;
         for (int b0 = 0; b0 < sd.n_owner_items; b0 += batch) {
             const int cnt = std::min(batch, sd.n_owner_items - b0);
             a.owner_order = sd.owner_order.p + b0;
             a.n_owners = cnt;
-            a.G = store ? g.G.p : g.wG.p;
-            a.g = store ? g.g.p : g.wg.p;
+            a.G = store ? sG : g.wG.p;
+            a.g = store ? sg : g.wg.p;
             a.corner = g.wcorner.p;
-            a.by_owner = store ? 1 : 0;
+            a.by_owner = store && !compact ? 1 : 0;
             MRB_CUDA(cudaMemsetAsync(g.counters.p, 0, sizeof(int), stream));
             const long long total = static_cast<long long>(cnt) * a.n_blocks;
             const int grid = static_cast<int>(std::min<long long>(static_cast<long long>(g.sms) * per_sm,
@@ -1201,11 +1322,12 @@ void AlsProblem::launch_half(bool user_side, cudaStream_t stream, int epilogue) 
     MRB_CUDA(cudaEventRecord(e0, stream));
     if (epilogue == EPI_STORE) {
         // rows without ratings are not in the work list: their blocks must read as zero
-        const size_t owners = user_side ? nu_ : ni_;
-        MRB_CUDA(cudaMemsetAsync(g.G.p, 0, sizeof(double) * owners * a.n * a.n, stream));
-        MRB_CUDA(cudaMemsetAsync(g.g.p, 0, sizeof(double) * owners * a.n, stream));
-        a.G_out = g.G.p;
-        a.g_out = g.g.p;
+        const size_t owners = compact ? sd.n_owner_items : (user_side ? nu_ : ni_);
+        a.G_out = compact ? g.oG.p : g.G.p;
+        a.g_out = compact ? g.og.p : g.g.p;
+        a.store_by_slot = compact ? 1 : 0;
+        MRB_CUDA(cudaMemsetAsync(a.G_out, 0, sizeof(double) * owners * a.n * a.n, stream));
+        MRB_CUDA(cudaMemsetAsync(a.g_out, 0, sizeof(double) * owners * a.n, stream));
         if (user_side) dispatch_gram<true, EPI_STORE>(a, g.sms, stream);
         else dispatch_gram<false, EPI_STORE>(a, g.sms, stream);
     } else {
@@ -1366,6 +1488,220 @@ static CgResult block_cg_solve(AlsProblem::GramState& g, double* x, int owners, 
     };
     // inside als() the inner solves always use (0.01, 200)            (matrix.cpp:818, 854-855)
     return native_cg_solve(apply, g.g.p, x, len, owners, 0.01, 200, ws, s);
+}
+
+
+// ---- algorithm 3 with rows dealt over several GPUs ----------------------------------------------
+// One CG half-sweep is driven phase by phase (cpp_ls_b200.h section 5, sharded.gram_cg_half_sweep):
+//
+//   begin (row) | B | RESIDUAL (chunk) | B | INIT (local) ; state
+//   [ MATVEC (row) | B | XR (chunk) | B | P (chunk) | B ] x batch ; state ...
+//   finish (chunk) | B
+//
+// B is a device barrier over all ranks (mrb_als_peer_barrier).  Row work of owner o is done by
+// the rank o is dealt to; vector work on element e by the rank owning chunk e / 256.  Every array
+// of the exchange block has one writer per element and phase, and the barriers make single
+// buffers enough:
+// * Ap (and g at begin) are stored by row owners into the chunk owner's block in begin / MATVEC
+//   and read by the chunk owner in RESIDUAL / XR, after the barrier; the next store is in the
+//   next MATVEC, after the barriers that follow XR.
+// * dots are stored into every block in MATVEC and summed in XR; the next store follows two
+//   barriers.  partials are stored into every block in RESIDUAL / XR and summed in INIT / P; the
+//   next store (XR) is behind the barrier after P and the one after MATVEC.
+// * p of element e is written by its chunk owner (RESIDUAL, P), locally and into the row owner's
+//   block; the row owner reads it in MATVEC after the barrier, the chunk owner in XR and P.  The
+//   next write (P) comes after the barrier that ends the MATVEC reading it.
+// * r, x (chunk range) and the CG state are local.  The scalar steps run on every rank over the
+//   same dots / partials arrays, so every rank reaches the same alpha, beta and stopping decision
+//   without communication.  finish stores the chunk range of x into every replica; the closing
+//   barrier makes the factors complete for the next half-sweep's Gram store.
+// Rows without ratings are in no work list: their Ap, g and dots stay +0.0 from cg_prepare, as the
+// one-GPU matvec computes them, and their x is updated by p = -0.0, i.e. left bit-unchanged.
+// Each element therefore sees the one-GPU operations in the one-GPU order, and every fixed-order
+// sum sees the one-GPU array: the factors, iteration counts and final_rr are those of one GPU.
+
+void AlsProblem::cg_prepare() {
+    ensure_gram();
+    GramState& g = *gram_;
+    if (g.xb.n) return;
+    const int n_u = k_ + 1, n_i = k_;
+    g.cg_user = cg_region(nu_, n_u, 0);
+    g.cg_item = cg_region(ni_, n_i, g.cg_user.end);
+    g.xb.alloc(g.cg_item.end);
+    MRB_CUDA(cudaMemsetAsync(g.xb.p, 0, sizeof(double) * g.xb.n, s_));
+    const size_t su = static_cast<size_t>(g.user.n_owner_items), si = static_cast<size_t>(g.item.n_owner_items);
+    g.oG.alloc(std::max<size_t>(std::max(su * n_u * n_u, si * n_i * n_i), 1));
+    g.og.alloc(std::max<size_t>(std::max(su * n_u, si * n_i), 1));
+    std::vector<int> ptr, ranks;
+    auto rank_map = [&](const int* d_ptr, int owners, DevBuf<int>& out) {
+        ptr.resize(static_cast<size_t>(owners) + 1);
+        ranks.assign(static_cast<size_t>(std::max(owners, 1)), -1);
+        MRB_CUDA(cudaMemcpyAsync(ptr.data(), d_ptr, sizeof(int) * ptr.size(), cudaMemcpyDeviceToHost, s_));
+        MRB_CUDA(cudaStreamSynchronize(s_));
+        owner_ranks_host(ptr.data(), owners, world_, ranks.data());
+        out.alloc(ranks.size());
+        out.upload(ranks.data(), ranks.size(), s_);
+        MRB_CUDA(cudaStreamSynchronize(s_));
+    };
+    rank_map(u_ptr_.p, nu_, g.user_rank);
+    rank_map(i_ptr_.p, ni_, g.item_rank);
+    g.xb_peers.assign(static_cast<size_t>(world_), nullptr);
+    g.xb_peers[static_cast<size_t>(rank_)] = g.xb.p;
+}
+
+double* AlsProblem::cg_exchange_block() {
+    MRB_REQUIRE(gram_ && gram_->xb.n, "als: cg_prepare has not been called");
+    return gram_->xb.p;
+}
+
+void AlsProblem::set_cg_peers(const std::vector<double*>& blocks) {
+    MRB_REQUIRE(gram_ && gram_->xb.n, "als: cg_prepare has not been called");
+    MRB_REQUIRE(static_cast<int>(blocks.size()) == world_, "als: one exchange block per rank");
+    gram_->xb_peers = blocks;
+    gram_->xb_peers[static_cast<size_t>(rank_)] = gram_->xb.p;
+}
+
+namespace {
+// one side's routing: every rank's arrays of the side, this rank's place, the chunk ranges
+CgRoute cg_route(const CgRegion& c, const std::vector<double*>& peers, const int* owner_rank,
+                 int rank, int world) {
+    CgRoute rt;
+    rt.owner_rank = owner_rank;
+    rt.n = c.n;
+    rt.rank = rank;
+    rt.world = world;
+    for (int q = 0; q <= world; q++) rt.chunk_lo[q] = cg_chunk_lo(c.vb, q, world);
+    for (int q = 0; q < world; q++) {
+        double* b = peers[static_cast<size_t>(q)];
+        rt.p[q] = b + c.p;
+        rt.Ap[q] = b + c.Ap;
+        rt.g[q] = b + c.g;
+        rt.dots[q] = b + c.dots;
+        rt.partials[q] = b + c.partials;
+    }
+    return rt;
+}
+
+template <int NPL>
+void launch_matvec_owned(const double* G, const double* g_c, const int* owner_order, int n_owned,
+                         const double* v, const CgRoute& rt, const CgState* guard, cudaStream_t s) {
+    const int mb = ceil_div(static_cast<long long>(n_owned) * 32, 256);
+    k_block_matvec_owned<NPL><<<mb, 256, 0, s>>>(G, g_c, owner_order, n_owned, v, rt, guard);
+    MRB_LAUNCHED(1);
+}
+}  // namespace
+
+// This rank's owned rows of the current side: Ap = G v into the chunk owners' blocks, dots into
+// every block (g_c: g along with Ap).
+void AlsProblem::cg_matvec(const double* v, const double* g_c, const CgState* guard, cudaStream_t s) {
+    GramState& g = *gram_;
+    const bool u = g.cg_on_user;
+    const Side& sd = u ? g.user : g.item;
+    const CgRegion& c = u ? g.cg_user : g.cg_item;
+    if (sd.n_owner_items == 0) return;
+    const CgRoute rt = cg_route(c, g.xb_peers, (u ? g.user_rank : g.item_rank).p, rank_, world_);
+    const int* oo = sd.owner_order.p;
+    const int m = sd.n_owner_items;
+    switch ((c.n + 31) / 32) {
+        case 1: launch_matvec_owned<1>(g.oG.p, g_c, oo, m, v, rt, guard, s); break;
+        case 2: launch_matvec_owned<2>(g.oG.p, g_c, oo, m, v, rt, guard, s); break;
+        case 3: launch_matvec_owned<3>(g.oG.p, g_c, oo, m, v, rt, guard, s); break;
+        case 4: launch_matvec_owned<4>(g.oG.p, g_c, oo, m, v, rt, guard, s); break;
+        case 5: launch_matvec_owned<5>(g.oG.p, g_c, oo, m, v, rt, guard, s); break;
+        default: throw Error(kErrArgument, "als algorithm 3: more than 160 unknowns per row");
+    }
+    MRB_CUDA(cudaGetLastError());
+}
+
+void AlsProblem::cg_begin(bool user_side, cudaStream_t stream) {
+    MRB_REQUIRE(gram_ && gram_->xb.n, "als: cg_prepare has not been called");
+    GramState& g = *gram_;
+    for (double* b : g.xb_peers)
+        MRB_REQUIRE(b != nullptr, "als: the exchange blocks of the peers are not set");
+    order_after_inputs(stream);
+    g.cg_on_user = user_side;
+    g.cg_begun = true;
+    launch_half(user_side, stream, EPI_STORE, true);
+    cg_matvec(user_side ? uf_.p : itf_.p, g.og.p, nullptr, stream);   // matrix.cpp:469-470
+}
+
+void AlsProblem::cg_phase(int phase, cudaStream_t s) {
+    MRB_REQUIRE(gram_ && gram_->cg_begun, "als: cg_begin has not been called");
+    GramState& g = *gram_;
+    const bool u = g.cg_on_user;
+    const CgRegion& c = u ? g.cg_user : g.cg_item;
+    double* b = g.xb.p;
+    CgState* st = reinterpret_cast<CgState*>(b + c.state);
+    double* total = b + c.partials + c.vb;
+    double* x = u ? uf_.p : itf_.p;
+    const CgRoute rt = cg_route(c, g.xb_peers, (u ? g.user_rank : g.item_rank).p, rank_, world_);
+    const int c0 = rt.chunk_lo[rank_], nc = rt.chunk_lo[rank_ + 1] - c0;
+    switch (phase) {
+        case CG_PHASE_RESIDUAL:                                                          // :472-476
+            if (nc > 0) {
+                k_bcg_residual<<<nc, 256, 0, s>>>(b + c.Ap, b + c.g, b + c.r, b + c.p, c.len,
+                                                  b + c.partials, c0, rt);
+                MRB_LAUNCHED(1);
+            }
+            break;
+        case CG_PHASE_INIT:                                                              // :485
+            k_bcg_sum<<<1, 1024, 0, s>>>(b + c.partials, c.vb, total, nullptr);
+            // inside als() the inner solves always use (0.01, 200)      (matrix.cpp:818, 854-855)
+            k_bcg_init<<<1, 1, 0, s>>>(st, total, 0.01, 200);
+            MRB_LAUNCHED(2);
+            break;
+        case CG_PHASE_MATVEC:                                                            // :493-494
+            cg_matvec(b + c.p, nullptr, st, s);
+            break;
+        case CG_PHASE_XR:
+            k_bcg_sum<<<1, 1024, 0, s>>>(b + c.dots, c.owners, total, st);              // :497
+            k_bcg_alpha<<<1, 1, 0, s>>>(st, total);                                      // :498
+            MRB_LAUNCHED(2);
+            if (nc > 0) {                                                                 // :501-504
+                k_bcg_update_xr<<<nc, 256, 0, s>>>(st, x, b + c.r, b + c.p, b + c.Ap, c.len,
+                                                   b + c.partials, c0, rt);
+                MRB_LAUNCHED(1);
+            }
+            break;
+        case CG_PHASE_P:
+            k_bcg_sum<<<1, 1024, 0, s>>>(b + c.partials, c.vb, total, st);              // :507
+            k_bcg_beta<<<1, 1, 0, s>>>(st, total);                                       // :510-518
+            MRB_LAUNCHED(2);
+            if (nc > 0) {                                                                 // :521
+                k_bcg_update_p<<<nc, 256, 0, s>>>(st, b + c.r, b + c.p, c.len, c0 * 256, rt);
+                MRB_LAUNCHED(1);
+            }
+            break;
+        default:
+            throw Error(kErrArgument, "als: unknown CG phase " + std::to_string(phase));
+    }
+    MRB_CUDA(cudaGetLastError());
+}
+
+CgState AlsProblem::cg_state(cudaStream_t s) {
+    MRB_REQUIRE(gram_ && gram_->cg_begun, "als: cg_begin has not been called");
+    GramState& g = *gram_;
+    const CgRegion& c = g.cg_on_user ? g.cg_user : g.cg_item;
+    CgState h;
+    MRB_CUDA(cudaMemcpyAsync(&h, g.xb.p + c.state, sizeof(CgState), cudaMemcpyDeviceToHost, s));
+    MRB_CUDA(cudaStreamSynchronize(s));
+    return h;
+}
+
+void AlsProblem::cg_finish(cudaStream_t s) {
+    MRB_REQUIRE(gram_ && gram_->cg_begun, "als: cg_begin has not been called");
+    GramState& g = *gram_;
+    const bool u = g.cg_on_user;
+    const CgRegion& c = u ? g.cg_user : g.cg_item;
+    PeerRows pr{};
+    set_peer_targets(pr, u ? uf_peers_ : itf_peers_, rank_);
+    const long long lo = static_cast<long long>(cg_chunk_lo(c.vb, rank_, world_)) * 256;
+    const long long hi = std::min<long long>(static_cast<long long>(cg_chunk_lo(c.vb, rank_ + 1, world_)) * 256, c.len);
+    g.cg_begun = false;
+    if (pr.n_peers == 0 || hi <= lo) return;
+    k_store_range<<<ceil_div(hi - lo, 256), 256, 0, s>>>(u ? uf_.p : itf_.p, lo, hi, pr);
+    MRB_LAUNCHED(1);
+    MRB_CUDA(cudaGetLastError());
 }
 
 }  // namespace mrb

@@ -506,6 +506,103 @@ int mrb_als_half_sweep(mrb_als_problem* p, int user_side, void* stream) {
     });
 }
 
+// ---- algorithm 3 (Gram block-CG) over the peer group
+int mrb_owner_ranks(const int* ptr, int owners, int world, int* out) {
+    return guarded([&] {
+        MRB_REQUIRE(ptr != nullptr && out != nullptr && owners >= 0 && world >= 1 && world <= PEER_MAX,
+                    "mrb_owner_ranks: bad arguments");
+        owner_ranks_host(ptr, owners, world, out);
+        return 0;
+    });
+}
+
+int mrb_als_cg_prepare(mrb_als_problem* p) {
+    return guarded([&] {
+        MRB_REQUIRE(p != nullptr, "null problem");
+        p->impl.cg_prepare();
+        return 0;
+    });
+}
+
+int mrb_als_cg_exchange_handle(mrb_als_problem* p, unsigned char* handle64) {
+    return guarded([&] {
+        MRB_REQUIRE(p != nullptr && handle64 != nullptr, "null argument");
+        ipc_export(p->impl.cg_exchange_block(), handle64);
+        return 0;
+    });
+}
+
+int mrb_als_cg_open_peers(mrb_als_problem* p, const unsigned char* handles_by_rank, int world) {
+    return guarded([&] {
+        MRB_REQUIRE(p != nullptr && handles_by_rank != nullptr && world == p->world,
+                    "mrb_als_cg_open_peers: bad arguments (one 64-byte handle per rank of the group)");
+        std::vector<double*> blocks(world, nullptr);
+        for (int r = 0; r < world; r++)
+            blocks[r] = r == p->rank ? p->impl.cg_exchange_block()
+                                     : static_cast<double*>(ipc_open_cached(handles_by_rank + 64 * static_cast<size_t>(r)));
+        p->impl.set_cg_peers(blocks);
+        return 0;
+    });
+}
+
+int mrb_als_cg_exchange_block(mrb_als_problem* p, void** d_block) {
+    return guarded([&] {
+        MRB_REQUIRE(p != nullptr && d_block != nullptr, "null argument");
+        *d_block = p->impl.cg_exchange_block();
+        return 0;
+    });
+}
+
+int mrb_als_cg_set_peer_pointers(mrb_als_problem* p, void* const* d_blocks, int world) {
+    return guarded([&] {
+        MRB_REQUIRE(p != nullptr && d_blocks != nullptr && world >= 1 && world <= PEER_MAX,
+                    "mrb_als_cg_set_peer_pointers: bad arguments");
+        std::vector<double*> blocks(world);
+        for (int r = 0; r < world; r++) blocks[r] = static_cast<double*>(d_blocks[r]);
+        p->impl.set_cg_peers(blocks);
+        return 0;
+    });
+}
+
+int mrb_als_cg_begin(mrb_als_problem* p, int user_side, void* stream) {
+    return guarded([&] {
+        MRB_REQUIRE(p != nullptr, "null problem");
+        p->impl.cg_begin(user_side != 0, static_cast<cudaStream_t>(stream));
+        return 0;
+    });
+}
+
+int mrb_als_cg_phase(mrb_als_problem* p, int phase, void* stream) {
+    return guarded([&] {
+        MRB_REQUIRE(p != nullptr, "null problem");
+        p->impl.cg_phase(phase, static_cast<cudaStream_t>(stream));
+        return 0;
+    });
+}
+
+int mrb_als_cg_state(mrb_als_problem* p, void* stream, int* done, int* iterations, double* final_rr) {
+    return guarded([&] {
+        MRB_REQUIRE(p != nullptr && done != nullptr && iterations != nullptr && final_rr != nullptr,
+                    "null argument");
+        const CgState h = p->impl.cg_state(static_cast<cudaStream_t>(stream));
+        *done = h.done;
+        *iterations = h.it;
+        *final_rr = h.final_rr;
+        if (peer_barrier_timed_out())
+            throw Error(kErrArgument, "a peer barrier timed out: a rank of the group did not arrive (" +
+                                          peer_barrier_timeout_report() + ")");
+        return 0;
+    });
+}
+
+int mrb_als_cg_finish(mrb_als_problem* p, void* stream) {
+    return guarded([&] {
+        MRB_REQUIRE(p != nullptr, "null problem");
+        p->impl.cg_finish(static_cast<cudaStream_t>(stream));
+        return 0;
+    });
+}
+
 int mrb_als_shard_sse(mrb_als_problem* p, void* stream, double* out) {
     return guarded([&] {
         MRB_REQUIRE(p != nullptr && out != nullptr, "null argument");

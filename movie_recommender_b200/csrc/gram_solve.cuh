@@ -28,7 +28,7 @@ struct WorkItem {
     int nseg;    // number of segments of the owner
     int slot;    // multi-segment owners: index of the owner's first partial buffer / counter id
     int multi;   // multi-segment owners: dense id (counter index), else -1
-    int pad;
+    int pad;     // position of the owner in the side's owner_order (its compact Gram slot)
 };
 
 MRB_DEVICE_INLINE void dmma884(double& c0, double& c1, double a, double b) {
@@ -61,6 +61,7 @@ struct GramArgs {
     int n_peers;              // number of entries of x_peers (0 on a single GPU)
     int debug_skip_solve;     // MRB_DEBUG_SKIP_SOLVE=1: time the accumulation alone (results invalid)
     int order_mode;           // how scheduler tickets map to the degree-sorted work list (work_index)
+    int store_by_slot;        // EPI_STORE: index G_out / g_out by WorkItem::pad (compact) instead of owner
 };
 
 // index of lower-triangular tile (ti, tj), tj <= ti

@@ -18,19 +18,54 @@ struct NativeCgWorkspace {
     CgState* state;         // device
 };
 
+// Routed stores of the sharded Gram block-CG (algorithm 3 over several GPUs, als_gram.cu).  Row
+// work (Gram store, block matvec) belongs to the rank the owner is dealt to; vector work belongs
+// to the rank that owns the element's 256-element chunk.  Every output element is stored where
+// its consumer reads it: p to the row owner, Ap / g to the chunk owner, the per-owner dots and
+// the per-chunk r.r partials to every rank.  Pointers are indexed by rank (entry `rank` is this
+// rank's own array).  The default (owner_rank == nullptr) routes nothing: one GPU.
+constexpr int CG_ROUTE_MAX = 8;
+struct CgRoute {
+    const int* owner_rank = nullptr;   // [owners] rank whose row work covers the owner, -1: no ratings
+    int n = 1;                         // unknowns per owner
+    int rank = 0, world = 0;
+    int chunk_lo[CG_ROUTE_MAX + 1] = {};   // rank r owns chunks chunk_lo[r] .. chunk_lo[r+1]-1
+    double* p[CG_ROUTE_MAX] = {};
+    double* Ap[CG_ROUTE_MAX] = {};
+    double* g[CG_ROUTE_MAX] = {};
+    double* dots[CG_ROUTE_MAX] = {};
+    double* partials[CG_ROUTE_MAX] = {};
+};
+
 namespace {
 
-// r = Ap - g, p = -r, per-CTA partial of r.r
+// The row owner's copy of p (sharded path; no-op without routing or when it is this rank).
+__device__ __forceinline__ void route_p(const CgRoute& rt, int i, double v) {
+    if (rt.owner_rank == nullptr) return;
+    const int o = rt.owner_rank[i / rt.n];
+    if (o >= 0 && o != rt.rank) rt.p[o][i] = v;
+}
+// Chunk c's r.r partial into the other ranks' partials arrays (sharded path).
+__device__ __forceinline__ void route_partial(const CgRoute& rt, int c, double v) {
+    for (int q = 0; q < rt.world; q++)
+        if (q != rt.rank) rt.partials[q][c] = v;
+}
+
+// r = Ap - g, p = -r, per-CTA partial of r.r.  CTA b works on chunk c0 + b (c0 = 0: all chunks
+// of a one-GPU launch; the sharded path launches this rank's chunk range).
 __global__ void __launch_bounds__(256)
 k_bcg_residual(const double* __restrict__ Ap, const double* __restrict__ g, double* __restrict__ r,
-               double* __restrict__ p, int len, double* __restrict__ partials) {
+               double* __restrict__ p, int len, double* __restrict__ partials, int c0 = 0,
+               const CgRoute route = CgRoute()) {
     __shared__ double red[256];
-    const int i = blockIdx.x * 256 + threadIdx.x;
+    const int c = c0 + blockIdx.x;
+    const int i = c * 256 + threadIdx.x;
     double s = 0;
     if (i < len) {
         const double ri = Ap[i] - g[i];
         r[i] = ri;
         p[i] = -ri;
+        route_p(route, i, -ri);
         s = ri * ri;
     }
     red[threadIdx.x] = s;
@@ -39,17 +74,21 @@ k_bcg_residual(const double* __restrict__ Ap, const double* __restrict__ g, doub
         if (threadIdx.x < off) red[threadIdx.x] += red[threadIdx.x + off];
         __syncthreads();
     }
-    if (threadIdx.x == 0) partials[blockIdx.x] = red[0];
+    if (threadIdx.x == 0) {
+        partials[c] = red[0];
+        route_partial(route, c, red[0]);
+    }
 }
 
-// x += alpha p, r += alpha Ap, per-CTA partial of the new r.r
+// x += alpha p, r += alpha Ap, per-CTA partial of the new r.r (chunks as k_bcg_residual)
 __global__ void __launch_bounds__(256)
 k_bcg_update_xr(const CgState* __restrict__ st, double* __restrict__ x, double* __restrict__ r,
                 const double* __restrict__ p, const double* __restrict__ Ap, int len,
-                double* __restrict__ partials) {
+                double* __restrict__ partials, int c0 = 0, const CgRoute route = CgRoute()) {
     if (st->done) return;
     __shared__ double red[256];
-    const int i = blockIdx.x * 256 + threadIdx.x;
+    const int c = c0 + blockIdx.x;
+    const int i = c * 256 + threadIdx.x;
     double s = 0;
     if (i < len) {
         const double a = st->alpha;
@@ -64,14 +103,23 @@ k_bcg_update_xr(const CgState* __restrict__ st, double* __restrict__ x, double* 
         if (threadIdx.x < off) red[threadIdx.x] += red[threadIdx.x + off];
         __syncthreads();
     }
-    if (threadIdx.x == 0) partials[blockIdx.x] = red[0];
+    if (threadIdx.x == 0) {
+        partials[c] = red[0];
+        route_partial(route, c, red[0]);
+    }
 }
 
+// p = beta p - r over elements i0 .. len-1 (i0 = 256 c0 in the sharded path)
 __global__ void k_bcg_update_p(const CgState* __restrict__ st, const double* __restrict__ r,
-                               double* __restrict__ p, int len) {
+                               double* __restrict__ p, int len, int i0 = 0,
+                               const CgRoute route = CgRoute()) {
     if (st->done) return;
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < len) p[i] = st->beta * p[i] - r[i];
+    const int i = i0 + blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < len) {
+        const double v = st->beta * p[i] - r[i];
+        p[i] = v;
+        route_p(route, i, v);
+    }
 }
 
 // guarded fixed-order sum (see k_sum_fixed)

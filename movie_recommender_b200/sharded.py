@@ -11,15 +11,68 @@ pointers (CUDA IPC mappings of the other ranks' buffers), i.e. the all-gather is
 producing kernel and overlaps the math row by row; between half-sweeps only a device-side flag
 barrier over the same mappings remains (``csrc/peer.cu``), enqueued on the stream -- no host
 round trip, no library collective.
+
+Algorithm 3 (the reference's CG on per-row Gram blocks) runs on the same partition: the rank a
+row is dealt to stores its Gram block and does its block matvec, the rank owning an element's
+256-element chunk does the vector updates, and the scalar steps run on every rank.  The results
+are bit-identical to one GPU (``gram_cg_half_sweep``, csrc/als_gram.cu).
 """
 import numpy as np
 
-from . import cpp_ls
+from . import _lib, cpp_ls
 
 
 def io_slice(n, rank, world):
-    """Contiguous 1/world share of n items that rank moves across its host link."""
+    """Contiguous 1/world share of n items that rank moves across its host link.  Also the
+    chunk range rank owns in the sharded CG: chunks io_slice(vb, rank, world) of a side's vb =
+    ceil(len / 256) chunks."""
     return n * rank // world, n * (rank + 1) // world
+
+
+# phases of one sharded CG half-sweep (MRB_CG_PHASE_* of include/cpp_ls_b200.h)
+CG_RESIDUAL, CG_INIT, CG_MATVEC, CG_XR, CG_P = range(5)
+CG_BATCH = 4   # guarded iterations between two reads of the CG state, as one-GPU algorithm 3
+
+
+def gram_cg_half_sweep(problems, user_side, stream, barrier, batch=CG_BATCH):
+    """One algorithm-3 half-sweep (Gram store, then the reference's CG) over the rows dealt to
+    each of ``problems`` -- the local ranks: one per process, or every rank of a group emulated in
+    one process on one stream.  ``barrier()`` separates the phases: a device barrier over the
+    group, or nothing where one stream already serialises the ranks.  Every rank's CG state is the
+    same, so every rank takes the same path and issues the same barrier sequence.  Returns
+    ``(iterations, final_rr)``."""
+    def each(call):
+        for p in problems:
+            call(p)
+
+    def state():
+        states = [p.cg_state(stream) for p in problems]
+        if any(s != states[0] for s in states[1:]):
+            raise RuntimeError("the ranks' CG states differ: %r" % (states,))
+        return states[0]
+
+    each(lambda p: p.cg_begin(user_side, stream))
+    barrier()
+    each(lambda p: p.cg_phase(CG_RESIDUAL, stream))
+    barrier()
+    each(lambda p: p.cg_phase(CG_INIT, stream))
+    done, iterations, final_rr = state()
+    while not done:
+        for _ in range(batch):
+            for phase in (CG_MATVEC, CG_XR, CG_P):
+                each(lambda p: p.cg_phase(phase, stream))
+                barrier()
+        done, iterations, final_rr = state()
+    each(lambda p: p.cg_finish(stream))
+    barrier()
+    return iterations, final_rr
+
+
+def relative_decrease(old_rr, rr):
+    """(old_rr - rr) / old_rr in IEEE arithmetic, as the C++ sweep loop computes it (0 / 0 is NaN,
+    which never stops the loop)."""
+    with np.errstate(all="ignore"):
+        return float(np.float64(old_rr - rr) / np.float64(old_rr))
 
 
 class ShardedAls:
@@ -94,6 +147,7 @@ class ShardedAls:
         # past it every replica holds the complete initial factors
         self.prob.peer_barrier(torch.cuda.current_stream().cuda_stream)
         marks.append(("ready", time.time()))
+        self._cg_ready = False   # the algorithm-3 exchange is set up by the first algorithm-3 call
         if rank == 0 and os.environ.get("MRB_E2E_TIMING"):
             import sys
             print("[ShardedAls] " + ", ".join("%s %.1f ms" % (marks[i][0], (marks[i][1] - marks[i - 1][1]) * 1e3)
@@ -102,7 +156,13 @@ class ShardedAls:
     def close(self):
         self.prob.close()
 
-    def sweep(self):
+    def sweep(self, algorithm=4):
+        """One sweep: algorithm 4 (exact half-sweeps) or 3 (Gram block-CG; returns the (iterations,
+        final_rr) of the user and of the item half-sweep)."""
+        if algorithm == 3:
+            return self._gram_cg_sweep()
+        if algorithm != 4:
+            raise ValueError("the sharded path implements algorithms 3 and 4")
         stream = self.torch.cuda.current_stream().cuda_stream
         # after each half-sweep the solved rows are already in every replica; the barrier waits
         # until every rank's kernel has finished
@@ -110,6 +170,54 @@ class ShardedAls:
         self.prob.peer_barrier(stream)
         self.prob.half_sweep(False, stream)
         self.prob.peer_barrier(stream)
+
+    def _cg_setup(self):
+        if self._cg_ready:
+            return
+        torch = self.torch
+        self.prob.cg_prepare()
+        mine = self.prob.cg_exchange_handle()
+        if self.world > 1:
+            t = torch.frombuffer(bytearray(mine), dtype=torch.uint8).to(self.device)
+            allh = torch.empty(64 * self.world, dtype=torch.uint8, device=self.device)
+            self.dist.all_gather_into_tensor(allh, t)
+            allh = bytes(allh.cpu().numpy())
+        else:
+            allh = mine
+        self.prob.cg_open_peers([allh[64 * r:64 * (r + 1)] for r in range(self.world)])
+        # no rank may store into a peer's exchange block before the peer has zeroed it
+        self.prob.peer_barrier(torch.cuda.current_stream().cuda_stream)
+        self._cg_ready = True
+
+    def _gram_cg_sweep(self):
+        self._cg_setup()
+        stream = self.torch.cuda.current_stream().cuda_stream
+
+        def barrier():
+            self.prob.peer_barrier(stream)
+        user = gram_cg_half_sweep([self.prob], True, stream, barrier)
+        item = gram_cg_half_sweep([self.prob], False, stream, barrier)
+        return user, item
+
+    def run(self, algorithm=3, min_r_decrease=0.01, max_iterations=200):
+        """Sweeps of algorithm 3 under the outer stopping rule of the one-GPU sweep loop
+        (matrix.cpp:871-875, on the item half-sweep's final_rr, which every rank holds); returns
+        an ``AlsRunInfo`` with sweeps_returned, sweeps_run, cg_iterations and last_rr."""
+        if algorithm != 3:
+            raise ValueError("ShardedAls.run drives algorithm 3; use sweep() for algorithm 4")
+        info = _lib.AlsRunInfo()
+        sweep, old_rr = 0, 0.0
+        while sweep < max_iterations:
+            (u_it, _), (i_it, rr) = self._gram_cg_sweep()
+            info.cg_iterations += u_it + i_it
+            info.sweeps_run += 1
+            info.last_rr = rr
+            if sweep >= 3 and relative_decrease(old_rr, rr) < min_r_decrease:
+                break
+            old_rr = rr
+            sweep += 1
+        info.sweeps_returned = sweep
+        return info
 
     def sse(self):
         """Training sum of squared errors after the last sweep, summed over ranks."""
