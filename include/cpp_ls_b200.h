@@ -286,7 +286,9 @@ MRB_API long long mrb_kernel_launches(void);
  *    python/full_data/build_similar_movies_db.py:21-221, works on co-rating vectors), so the
  *    arithmetic is defined by oracle/ls_oracle.c:oracle_cosine_topk and met bit-exactly:
  *    row-normalised fp64 factors, sequential sums, top-k by (score desc, id asc), self excluded.
- *    Queries q_lo..q_hi-1 only: the multi-GPU split is by query block.
+ *    Queries q_lo..q_hi-1 only: the multi-GPU split is by query block.  num_factors 1..160
+ *    (every rank the exact ALS solvers train; 1..64 with MRB_SIM_KERNEL=dmma), topk 1..56;
+ *    anything else is refused with MRB_ERR_ARGUMENT.
  * ---------------------------------------------------------------------------------------- */
 typedef struct mrb_sim_info {
     float candidates_ms;   /* normalisation + tensor-core GEMM fused with candidate selection */

@@ -54,7 +54,8 @@ __device__ __forceinline__ bool precedes(double sa, int ia, double sb, int ib) {
     return sa > sb || (sa == sb && ia < ib);
 }
 
-// Row norms and normalised rows in the oracle's arithmetic; Hp = zero-padded copy, row stride kp.
+// Row norms and normalised rows in the oracle's arithmetic, all k columns; Hp (the fp64 kernel's
+// operand, nullptr otherwise) = zero-padded copy, row stride kp >= k.
 __global__ void k_sim_normalize(const double* __restrict__ M, int n, int k, int kp,
                                 double* __restrict__ H, double* __restrict__ Hp) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -63,11 +64,9 @@ __global__ void k_sim_normalize(const double* __restrict__ M, int n, int k, int 
     double s = 0;
     for (int f = 0; f < k; f++) s = __dadd_rn(s, __dmul_rn(m[f], m[f]));
     const double nrm = sqrt(s);
-    for (int f = 0; f < kp; f++) {
-        const double v = (f < k && nrm > 0) ? m[f] / nrm : 0.0;
-        if (f < k) H[static_cast<size_t>(i) * k + f] = v;
-        Hp[static_cast<size_t>(i) * kp + f] = v;
-    }
+    for (int f = 0; f < k; f++) H[static_cast<size_t>(i) * k + f] = nrm > 0 ? m[f] / nrm : 0.0;
+    if (Hp != nullptr)
+        for (int f = 0; f < kp; f++) Hp[static_cast<size_t>(i) * kp + f] = (f < k && nrm > 0) ? m[f] / nrm : 0.0;
 }
 
 struct SimSmem {
@@ -323,7 +322,7 @@ k_sim_rescore(const double* __restrict__ H, int n, int k, int topk, int q_lo, in
         scores_out[static_cast<size_t>(w) * topk + r] = 0.0;
     }
     // Every dropped movie has approximate score <= cand_thr, hence exact score <= cand_thr + eps
-    // (eps = the candidate GEMM's error bound: 1e-12 for the fp64 path, SIM_TC_EPS for tf32).
+    // (eps = the candidate GEMM's error bound: 1e-12 for the fp64 path, sim_tc_eps(k) for tf32).
     // It cannot belong to the top-k if the exact k-th score is clearly above that.
     const bool certified = cnt < SIM_C || kth - cand_thr[w] > eps;
     if (lane == 0) flags[w] = certified ? 0 : 1;
@@ -471,22 +470,9 @@ void launch_candidates(const double* Hp, int n, int q_lo, int q_hi, int* cand_id
 
 SimResult cosine_topk(const double* M, int n, int k, int topk, int q_lo, int q_hi, int* ids_out,
                       double* scores_out) {
-    MRB_REQUIRE(n >= 0 && k >= 1 && k <= 64, "cosine_topk: factor count must be in 1..64");
+    MRB_REQUIRE(n >= 0 && k >= 1 && k <= 160, "cosine_topk: factor count must be in 1..160");
     MRB_REQUIRE(topk >= 1 && topk <= SIM_C - 8, "cosine_topk: topk must be in 1..56");
     MRB_REQUIRE(q_lo >= 0 && q_lo <= q_hi && q_hi <= n, "cosine_topk: bad query range");
-    SimResult res;
-    const int nq = q_hi - q_lo;
-    if (nq == 0) return res;
-    // supported k-step counts (factor count padded with zeros to 4 KS)
-    const int ks_needed = (k + 3) / 4;
-    const int ks = ks_needed <= 4 ? 4 : ks_needed <= 8 ? 8 : ks_needed <= 13 ? 13 : 16;
-    const int kp = ks * 4;
-    cudaStream_t s;
-    MRB_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-    struct StreamGuard { cudaStream_t s; ~StreamGuard() { cudaStreamDestroy(s); } } sg{s};
-    DevBuf<double> d_M(static_cast<size_t>(n) * k), H(static_cast<size_t>(n) * k),
-        Hp(static_cast<size_t>(n) * kp + 16);
-    d_M.upload(M, static_cast<size_t>(n) * k, s);
     // MRB_SIM_KERNEL=dmma selects the fp64 mma.sync candidate kernel (the round-1 path, kept as
     // the A/B baseline); the default is the tcgen05 / TMA / TMEM kernel of similarity_tc.cu --
     // two passes with a fixed per-row threshold for catalogues of 128 ... 512 tiles
@@ -494,9 +480,25 @@ SimResult cosine_topk(const double* M, int n, int k, int topk, int q_lo, int q_h
     const char* which = std::getenv("MRB_SIM_KERNEL");
     const std::string mode = which != nullptr ? which : "";
     const bool use_dmma = mode == "dmma";
+    // the fp64 kernel's double-buffered stage (2 x 128 rows x kp doubles) fits beside its
+    // candidate lists only up to 64 factors
+    MRB_REQUIRE(!use_dmma || k <= 64, "cosine_topk: MRB_SIM_KERNEL=dmma takes a factor count in 1..64");
+    SimResult res;
+    const int nq = q_hi - q_lo;
+    if (nq == 0) return res;
+    // supported k-step counts of the fp64 kernel (factor count padded with zeros to 4 KS)
+    const int ks_needed = (k + 3) / 4;
+    const int ks = ks_needed <= 4 ? 4 : ks_needed <= 8 ? 8 : ks_needed <= 13 ? 13 : 16;
+    const int kp = ks * 4;
+    cudaStream_t s;
+    MRB_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+    struct StreamGuard { cudaStream_t s; ~StreamGuard() { cudaStreamDestroy(s); } } sg{s};
+    DevBuf<double> d_M(static_cast<size_t>(n) * k), H(static_cast<size_t>(n) * k),
+        Hp(use_dmma ? static_cast<size_t>(n) * kp + 16 : 0);     // Hp.p == nullptr on the tcgen05 path
+    d_M.upload(M, static_cast<size_t>(n) * k, s);
     const bool two_pass = !use_dmma && mode != "tc1" && sim_tc_twopass_applies(n);
     const int cap = two_pass ? sim_tc_twopass_capacity() : SIM_C;
-    const double eps = use_dmma ? 1e-12 : SIM_TC_EPS;
+    const double eps = use_dmma ? 1e-12 : sim_tc_eps(k);
     DevBuf<int> cand_id(static_cast<size_t>(nq) * cap), flags(nq);
     DevBuf<int> cand_cnt(static_cast<size_t>(nq) * (two_pass ? sim_tc_twopass_groups() : 1));
     DevBuf<double> cand_thr(nq);

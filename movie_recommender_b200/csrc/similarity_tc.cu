@@ -1,22 +1,34 @@
 // K5, phase A on the 5th-generation tensor cores: the candidate GEMM  S ~ Mhat Mhat^T  as
 // tcgen05.mma (kind::tf32, operands in shared memory via TMA, accumulators in tensor memory)
 // fused with the per-row candidate selection, which reads the accumulators straight out of TMEM
-// (tcgen05.ld).  The N x N score matrix never exists.
+// (tcgen05.ld).  The N x N score matrix never exists.  1 ... 160 factors.
 //
 // Why tf32 is enough: the candidates are only a SUPERSET filter.  Phase B (similarity.cu) re-scores
-// the 64 candidates of every query in the oracle's exact fp64 summation order and certifies the
-// result against the approximate threshold: |S_tf32 - S_exact| <= (2^-10 + 2^-22) sum |a_i b_i| +
-// fp32 accumulation <= 1.0e-3 for unit rows (both operands rounded to nearest tf32, 11 significant
-// bits; Cauchy-Schwarz), so a dropped movie can only belong to the top-k if the exact k-th score
-// is within 1.0e-3 of the approximate 64th -- those queries (rare: 14 spare candidates) are
-// recomputed exhaustively (phase C).  ids and scores stay bit-exact against oracle_cosine_topk.
+// the candidates of every query in the oracle's exact fp64 summation order and certifies the
+// result against the approximate threshold widened by eps = sim_tc_eps(Kp), a bound on
+// |S_tf32 - S_exact| for unit rows at the executed contraction length Kp = 8 ceil(k / 8):
+//   operands  each factor is rounded fp64 -> fp32 -> tf32 (nearest, 11 significant bits), a
+//             relative error u <= 2^-11 + 2^-24; a product of two carries <= 2u + u^2, and
+//             sum |a_i b_i| <= |a| |b| = 1 (Cauchy-Schwarz), so <= 2^-10 + 2^-21 in all;
+//   fp32 sum  the tensor core's accumulation order and rounding are not documented.  Assume the
+//             worst of truncation: every one of the Kp additions loses up to 2 units in the last
+//             place of a partial sum bounded by sum |a_i b_i| <= 1 (one for aligning the addend,
+//             one for the result), <= Kp 2^-22.
+// eps(Kp) = 2^-10 + 2^-21 + Kp 2^-22: 9.92e-4 at Kp = 64, 1.0076e-3 at 128, 1.0152e-3 at 160.
+// For Kp <= 96 it stays below SIM_TC_EPS = 1.0e-3, which is used there unchanged.  A dropped
+// movie can only belong to the top-k if the exact k-th score is within eps of the approximate
+// 64th -- those queries (rare: 14 spare candidates) are recomputed exhaustively (phase C).  A
+// wider eps only sends more queries there; ids and scores stay bit-exact against
+// oracle_cosine_topk.
 //
 // One CTA per 128 query rows (one per SM, persistent over the catalogue):
-//   warp 0    TMA producer: the query tile once, then the catalogue in tiles of 128 rows x 64
-//             (two 128-byte-swizzled K blocks of 32 tf32) through a 2-stage mbarrier ring
-//   warp 1    MMA issuer: 7 x tcgen05.mma m128 n128 k8 per tile (K = 50 padded to 56) into one of
-//             4 accumulator buffers (128 lanes x 128 columns fp32 each = all 512 TMEM columns);
-//             tcgen05.commit frees the smem stage and publishes the accumulator
+//   warp 0    TMA producer: the query tile once (KB K blocks of 128 rows x 32 tf32, one
+//             128-byte swizzle row each, KB = max(2, ceil(k / 32))), then the catalogue as
+//             (tile of 128 rows, K block) pairs through an mbarrier ring of 16 KB K-block stages
+//   warp 1    MMA issuer: per K block up to 4 x tcgen05.mma m128 n128 k8 (ceil(k / 8) per tile,
+//             K = 50 padded to 56) into one of 4 accumulator buffers (128 lanes x 128 columns
+//             fp32 each = all 512 TMEM columns); tcgen05.commit frees each K-block stage as soon
+//             as its MMAs have read it, and publishes the accumulator after the tile's last block
 //   warps 2-5 epilogue: thread = query row = TMEM lane; 16 scores per tcgen05.ld (the next load in
 //             flight while the current chunk is examined); per score one compare against the
 //             row's threshold and one warp vote -- ~430 of 53 889 scores per row ever pass, but
@@ -25,6 +37,8 @@
 //             memory (the row belongs to the thread: no atomics); a buffer that could overflow is
 //             merged into the sorted 64-entry list by the whole warp (bitonic sort + merge in
 //             registers), which raises the threshold.
+// Shared memory at KB = 5, one pass (the tight case): query tile 5 x 16 KB + per-row lists 96 KB +
+// 3 ring stages x 16 KB + barriers = 230 400 bytes, + 1 KB alignment slack <= 232 448.
 #include <cuda.h>
 
 #include <algorithm>
@@ -37,9 +51,8 @@ namespace {
 
 constexpr int TC_M = 128;          // query rows per CTA
 constexpr int TC_N = 128;          // catalogue rows per tile
-constexpr int TC_KB = 32;          // tf32 per 128-byte swizzle row
-constexpr int TC_KP = 64;          // padded factor count (two K blocks)
-constexpr int TC_STAGES = 2;
+constexpr int TC_KB = 32;          // tf32 per 128-byte swizzle row (one K block)
+constexpr int TC_KMAX = 160;       // factor limit: 5 K blocks
 constexpr int TC_ACC = 4;          // accumulator buffers in TMEM
 constexpr int TC_C = 64;           // candidates kept per query (== SIM_C of similarity.cu)
 constexpr int TC_PEND = 32;        // pending buffer per query
@@ -51,20 +64,26 @@ constexpr int TC_PEND = 32;        // pending buffer per query
 template <int MODE> constexpr int tc_sets() { return MODE == 0 ? 1 : 4; }
 template <int MODE> constexpr int tc_threads() { return 64 + 128 * tc_sets<MODE>(); }
 constexpr int TC_TILE_BYTES = TC_N * TC_KB * 4;          // one K block of one tile: 16 KB
+constexpr int TC_SMEM_MAX = 232448;                      // opt-in shared memory per CTA
 
-// MODE_TOPK keeps the per-row candidate lists in shared memory (2 catalogue stages fit beside
-// them); the two-pass modes keep nothing per row and use the room for a deeper TMA ring.
 enum { MODE_TOPK = 0, MODE_TILEMAX = 1, MODE_COLLECT = 2 };
+// K-block stages of the catalogue ring.  MODE_TOPK keeps 96 KB of per-row candidate lists in
+// shared memory and takes what fits beside them and the KB-block query tile (4 at KB = 2, as many
+// as fit into 224 KB); the two-pass modes keep nothing per row and run 8 stages (128 KB in
+// flight) at every KB.
+template <int MODE, int KB> constexpr int tc_stages() {
+    return MODE != MODE_TOPK ? 8 : KB == 2 ? 4 : KB == 3 ? 5 : KB == 4 ? 4 : 3;
+}
 constexpr int TC_SETS2 = 4;        // epilogue warp groups of the two-pass modes (= column groups per tile)
 constexpr int TC_CAPS = 48;        // candidate capacity per (query, column group): ~17 expected
 constexpr int TC_CAP2 = TC_SETS2 * TC_CAPS;
 
-template <int MODE>
+template <int MODE, int KB>
 struct TcSmemT {
-    static constexpr int STAGES = MODE == MODE_TOPK ? TC_STAGES : 4;
+    static constexpr int STAGES = tc_stages<MODE, KB>();
     static constexpr int LROWS = MODE == MODE_TOPK ? TC_M : 1;
-    alignas(1024) float a[2][TC_M * TC_KB];              // query tile, two K blocks
-    alignas(1024) float b[STAGES][2][TC_N * TC_KB];      // catalogue stages
+    alignas(1024) float a[KB][TC_M * TC_KB];             // query tile, KB K blocks
+    alignas(1024) float b[STAGES][TC_N * TC_KB];         // catalogue ring, one K block per stage
     float score[LROWS][TC_C + TC_PEND];                  // [0,64) sorted list, [64,96) pending
     int id[LROWS][TC_C + TC_PEND];
     unsigned long long full_bar[STAGES], empty_bar[STAGES];
@@ -72,7 +91,6 @@ struct TcSmemT {
     unsigned long long a_bar;
     unsigned tmem_base;
 };
-using TcSmem = TcSmemT<MODE_TOPK>;
 
 __device__ __forceinline__ unsigned smem_u32(const void* p) {
     return static_cast<unsigned>(__cvta_generic_to_shared(p));
@@ -176,7 +194,8 @@ __device__ __forceinline__ FKV fkv_pick(const FKV& a, const FKV& b, bool keep_fi
 // Whole-warp merge of one row's pending buffer (pc <= 32 entries) into its sorted list (lc <= 64):
 // bitonic sort of the pending entries across the lanes, one compare step against the list tail
 // (list[32 + i] vs pending[31 - i] keeps the best 64 as a bitonic sequence), bitonic merge of 64.
-__device__ __forceinline__ void tc_merge_row(TcSmem& sm, int row, int lc, int pc, int lane) {
+template <class Smem>
+__device__ __forceinline__ void tc_merge_row(Smem& sm, int row, int lc, int pc, int lane) {
     const FKV worst = {-3.0e38f, 0x7fffffff};
     FKV b = lane < pc ? FKV{sm.score[row][TC_C + lane], sm.id[row][TC_C + lane]} : worst;
     FKV a0 = lane < lc ? FKV{sm.score[row][lane], sm.id[row][lane]} : worst;
@@ -216,12 +235,12 @@ __device__ __forceinline__ void tc_merge_row(TcSmem& sm, int row, int lc, int pc
 //              reaches it (~70 per row) to the row's list in global memory -- no sorting, no
 //              merging, no moving threshold in the hot loop.  The GEMM runs twice; it is the
 //              cheap part.
-template <int MODE>
+template <int MODE, int KB>
 __global__ void __launch_bounds__(tc_threads<MODE>(), 1)
 k_sim_tc(const __grid_constant__ CUtensorMap map, int n, int ksteps, int q_lo, int q_hi,
          int* __restrict__ cand_id, double* __restrict__ cand_thr, int* __restrict__ cand_cnt,
          float* __restrict__ tile_max, int rows_pad, const float* __restrict__ thr0) {
-    using Smem = TcSmemT<MODE>;
+    using Smem = TcSmemT<MODE, KB>;
     constexpr int STAGES = Smem::STAGES;
     extern __shared__ unsigned char smem_raw[];
     Smem& sm = *reinterpret_cast<Smem*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -248,15 +267,14 @@ k_sim_tc(const __grid_constant__ CUtensorMap map, int n, int ksteps, int q_lo, i
     if (warp == 0) {
         // ================= TMA producer =================
         if (lane == 0) {
-            mbar_expect_tx(&sm.a_bar, 2 * TC_TILE_BYTES);
-            tma_load_2d(sm.a[0], &map, 0, q_base, &sm.a_bar);
-            tma_load_2d(sm.a[1], &map, TC_KB, q_base, &sm.a_bar);
-            for (int t = 0; t < ntiles; t++) {
-                const int s = t % STAGES;
-                if (t >= STAGES) mbar_wait(&sm.empty_bar[s], ((t / STAGES) - 1) & 1);
-                mbar_expect_tx(&sm.full_bar[s], 2 * TC_TILE_BYTES);
-                tma_load_2d(sm.b[s][0], &map, 0, t * TC_N, &sm.full_bar[s]);
-                tma_load_2d(sm.b[s][1], &map, TC_KB, t * TC_N, &sm.full_bar[s]);
+            mbar_expect_tx(&sm.a_bar, KB * TC_TILE_BYTES);
+            for (int kb = 0; kb < KB; kb++) tma_load_2d(sm.a[kb], &map, kb * TC_KB, q_base, &sm.a_bar);
+            // step i = t KB + kb carries K block kb of catalogue tile t
+            for (int i = 0; i < ntiles * KB; i++) {
+                const int s = i % STAGES, t = i / KB, kb = i % KB;
+                if (i >= STAGES) mbar_wait(&sm.empty_bar[s], ((i / STAGES) - 1) & 1);
+                mbar_expect_tx(&sm.full_bar[s], TC_TILE_BYTES);
+                tma_load_2d(sm.b[s], &map, kb * TC_KB, t * TC_N, &sm.full_bar[s]);
             }
         }
     } else if (warp == 1) {
@@ -264,17 +282,20 @@ k_sim_tc(const __grid_constant__ CUtensorMap map, int n, int ksteps, int q_lo, i
         if (lane == 0) {
             mbar_wait(&sm.a_bar, 0);
             for (int t = 0; t < ntiles; t++) {
-                const int s = t % STAGES, a = t % TC_ACC;
+                const int a = t % TC_ACC;
                 if (t >= TC_ACC) mbar_wait(&sm.acc_empty[a], ((t / TC_ACC) - 1) & 1);
-                mbar_wait(&sm.full_bar[s], (t / STAGES) & 1);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 const unsigned d = tmem + a * TC_N;
-                for (int ks = 0; ks < ksteps; ks++) {
-                    const int kb = ks >> 2, off = (ks & 3) * 32;     // 8 tf32 = 32 bytes per k-step
-                    umma_tf32(d, umma_desc(sm.a[kb], off), umma_desc(sm.b[s][kb], off), ks > 0);
+                for (int kb = 0; kb < KB; kb++) {
+                    const int i = t * KB + kb, s = i % STAGES;
+                    mbar_wait(&sm.full_bar[s], (i / STAGES) & 1);
+                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    for (int ks = 4 * kb; ks < min(ksteps, 4 * kb + 4); ks++) {
+                        const int off = (ks & 3) * 32;              // 8 tf32 = 32 bytes per k-step
+                        umma_tf32(d, umma_desc(sm.a[kb], off), umma_desc(sm.b[s], off), ks > 0);
+                    }
+                    umma_commit(&sm.empty_bar[s]);  // stage free once these MMAs have read it
                 }
-                umma_commit(&sm.empty_bar[s]);     // smem stage free once these MMAs have read it
-                umma_commit(&sm.acc_full[a]);      // accumulator complete
+                umma_commit(&sm.acc_full[a]);       // accumulator complete
             }
         }
     } else {
@@ -450,12 +471,13 @@ k_sim_tc(const __grid_constant__ CUtensorMap map, int n, int ksteps, int q_lo, i
     }
 }
 
-// Hq[row][f] = tf32(Mhat[row][f]) as fp32 bits (round to nearest), zero beyond k and beyond n
-__global__ void k_sim_to_tf32(const double* __restrict__ H, int n, int k, int rows_padded,
+// Hq[row][f] = tf32(Mhat[row][f]) as fp32 bits (round to nearest), zero beyond k and beyond n;
+// row stride kp = KB * 32
+__global__ void k_sim_to_tf32(const double* __restrict__ H, int n, int k, int kp, int rows_padded,
                               float* __restrict__ Hq) {
     const size_t e = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-    if (e >= static_cast<size_t>(rows_padded) * TC_KP) return;
-    const int row = static_cast<int>(e / TC_KP), f = static_cast<int>(e % TC_KP);
+    if (e >= static_cast<size_t>(rows_padded) * kp) return;
+    const int row = static_cast<int>(e / kp), f = static_cast<int>(e % kp);
     float x = (row < n && f < k) ? static_cast<float>(H[static_cast<size_t>(row) * k + f]) : 0.0f;
     unsigned u;
     asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(x));
@@ -532,51 +554,72 @@ k_sim_select_thr(const float* __restrict__ tile_max, int ntiles, int sets, int r
     }
 }
 
-template <int MODE>
+template <int MODE, int KB>
 void launch_tc(const CUtensorMap& map, int grid, int n, int ksteps, int q_lo, int q_hi, int* cand_id,
                double* cand_thr, int* cand_cnt, float* tile_max, int rows_pad, const float* thr0,
                cudaStream_t s) {
-    const size_t smem = sizeof(TcSmemT<MODE>) + 1024;
+    const size_t smem = sizeof(TcSmemT<MODE, KB>) + 1024;      // + slack for the 1024-byte alignment
+    static_assert(sizeof(TcSmemT<MODE, KB>) + 1024 <= TC_SMEM_MAX, "k_sim_tc: shared memory over the limit");
     static bool attr = false;
     if (!attr) {
-        MRB_CUDA(cudaFuncSetAttribute(k_sim_tc<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        MRB_CUDA(cudaFuncSetAttribute(k_sim_tc<MODE, KB>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       static_cast<int>(smem)));
         attr = true;
     }
-    k_sim_tc<MODE><<<grid, tc_threads<MODE>(), smem, s>>>(map, n, ksteps, q_lo, q_hi, cand_id, cand_thr, cand_cnt,
-                                                  tile_max, rows_pad, thr0);
+    k_sim_tc<MODE, KB><<<grid, tc_threads<MODE>(), smem, s>>>(map, n, ksteps, q_lo, q_hi, cand_id, cand_thr,
+                                                              cand_cnt, tile_max, rows_pad, thr0);
     MRB_LAUNCHED(1);
     MRB_CUDA(cudaGetLastError());
+}
+
+template <int KB>
+void candidates_tc(const CUtensorMap& map, int grid, int n, int ksteps, int q_lo, int q_hi, int* cand_id,
+                   double* cand_thr, int* cand_cnt, cudaStream_t s, bool two_pass) {
+    if (!two_pass) {
+        launch_tc<MODE_TOPK, KB>(map, grid, n, ksteps, q_lo, q_hi, cand_id, cand_thr, cand_cnt, nullptr, 0, nullptr,
+                                 s);
+        return;
+    }
+    const int nq = q_hi - q_lo, ntiles = ceil_div(n, TC_N), rows_pad = grid * TC_M;
+    DevBuf<float> tile_max(static_cast<size_t>(ntiles) * TC_SETS2 * rows_pad), thr0(nq);
+    launch_tc<MODE_TILEMAX, KB>(map, grid, n, ksteps, q_lo, q_hi, nullptr, nullptr, nullptr, tile_max.p, rows_pad,
+                                nullptr, s);
+    k_sim_select_thr<<<ceil_div(static_cast<long long>(nq) * 32, 256), 256, 0, s>>>(tile_max.p, ntiles, TC_SETS2,
+                                                                                  rows_pad, nq, TC_C, thr0.p);
+    MRB_LAUNCHED(1);
+    launch_tc<MODE_COLLECT, KB>(map, grid, n, ksteps, q_lo, q_hi, cand_id, cand_thr, cand_cnt, nullptr, rows_pad,
+                                thr0.p, s);
+    MRB_CUDA(cudaStreamSynchronize(s));   // tile_max / thr0 are released on return
 }
 
 }  // namespace
 
 int sim_tc_candidates() { return TC_C; }
-int sim_tc_padded_k() { return TC_KP; }
 int sim_tc_twopass_capacity() { return TC_CAP2; }
 int sim_tc_twopass_groups() { return TC_SETS2; }
 // the two-pass path needs at least 2 x 64 tile maxima per row for its threshold to be tight
 bool sim_tc_twopass_applies(int n) { return (n + TC_N - 1) / TC_N >= 128 && (n + TC_N - 1) / TC_N <= 512; }
 
-// H: device, n x k normalised rows (fp64).
+// H: device, n x k normalised rows (fp64), 1 <= k <= 160.
 // one pass (two_pass == false): cand_id[nq][64], cand_thr[nq] = approximate 64th score, cand_cnt[nq];
 // two passes: cand_id[nq][128] = every column whose approximate score reaches cand_thr[nq] (a lower
 // bound of the row's 64th largest approximate score), cand_cnt[nq] (may exceed 128: overflow).
 void cosine_candidates_tc(const double* d_H, int n, int k, int q_lo, int q_hi, int* cand_id,
                           double* cand_thr, int* cand_cnt, cudaStream_t s, bool two_pass) {
-    MRB_REQUIRE(k >= 1 && k <= TC_KP, "cosine_candidates_tc: factor count must be in 1..64");
+    MRB_REQUIRE(k >= 1 && k <= TC_KMAX, "cosine_candidates_tc: factor count must be in 1..160");
     const int nq = q_hi - q_lo;
     if (nq <= 0) return;
     const int grid = ceil_div(nq, TC_M);
+    const int kb = std::max(2, ceil_div(k, TC_KB)), kp = kb * TC_KB;   // K blocks, row width of Hq
     // rows the TMA may touch: the catalogue tiles and the last query tile (out-of-bounds rows read 0)
     const int rows_padded = std::max(ceil_div(n, TC_N) * TC_N, q_lo + grid * TC_M);
-    DevBuf<float> Hq(static_cast<size_t>(rows_padded) * TC_KP);
-    const size_t total = static_cast<size_t>(rows_padded) * TC_KP;
-    k_sim_to_tf32<<<ceil_div(static_cast<long long>(total), 256), 256, 0, s>>>(d_H, n, k, rows_padded, Hq.p);
+    const size_t total = static_cast<size_t>(rows_padded) * kp;
+    DevBuf<float> Hq(total);
+    k_sim_to_tf32<<<ceil_div(static_cast<long long>(total), 256), 256, 0, s>>>(d_H, n, k, kp, rows_padded, Hq.p);
     MRB_LAUNCHED(1);
     CUtensorMap map;
-    const cuuint64_t dims[2] = {static_cast<cuuint64_t>(TC_KP), static_cast<cuuint64_t>(rows_padded)};
-    const cuuint64_t strides[1] = {static_cast<cuuint64_t>(TC_KP) * sizeof(float)};
+    const cuuint64_t dims[2] = {static_cast<cuuint64_t>(kp), static_cast<cuuint64_t>(rows_padded)};
+    const cuuint64_t strides[1] = {static_cast<cuuint64_t>(kp) * sizeof(float)};
     const cuuint32_t box[2] = {TC_KB, TC_N};
     const cuuint32_t estr[2] = {1, 1};
     const CUresult rc = encode_tiled()(&map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, Hq.p, dims, strides, box, estr,
@@ -584,19 +627,11 @@ void cosine_candidates_tc(const double* d_H, int n, int k, int q_lo, int q_hi, i
                                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     MRB_REQUIRE(rc == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed");
     const int ksteps = (k + 7) / 8;
-    if (!two_pass) {
-        launch_tc<MODE_TOPK>(map, grid, n, ksteps, q_lo, q_hi, cand_id, cand_thr, cand_cnt, nullptr, 0, nullptr, s);
-    } else {
-        const int ntiles = ceil_div(n, TC_N), rows_pad = grid * TC_M;
-        DevBuf<float> tile_max(static_cast<size_t>(ntiles) * TC_SETS2 * rows_pad), thr0(nq);
-        launch_tc<MODE_TILEMAX>(map, grid, n, ksteps, q_lo, q_hi, nullptr, nullptr, nullptr, tile_max.p, rows_pad,
-                                nullptr, s);
-        k_sim_select_thr<<<ceil_div(static_cast<long long>(nq) * 32, 256), 256, 0, s>>>(tile_max.p, ntiles, TC_SETS2,
-                                                                                      rows_pad, nq, TC_C, thr0.p);
-        MRB_LAUNCHED(1);
-        launch_tc<MODE_COLLECT>(map, grid, n, ksteps, q_lo, q_hi, cand_id, cand_thr, cand_cnt, nullptr, rows_pad,
-                                thr0.p, s);
-        MRB_CUDA(cudaStreamSynchronize(s));   // tile_max / thr0 are released on return
+    switch (kb) {
+        case 2: candidates_tc<2>(map, grid, n, ksteps, q_lo, q_hi, cand_id, cand_thr, cand_cnt, s, two_pass); break;
+        case 3: candidates_tc<3>(map, grid, n, ksteps, q_lo, q_hi, cand_id, cand_thr, cand_cnt, s, two_pass); break;
+        case 4: candidates_tc<4>(map, grid, n, ksteps, q_lo, q_hi, cand_id, cand_thr, cand_cnt, s, two_pass); break;
+        default: candidates_tc<5>(map, grid, n, ksteps, q_lo, q_hi, cand_id, cand_thr, cand_cnt, s, two_pass); break;
     }
     MRB_CUDA(cudaStreamSynchronize(s));   // Hq is released on return
 }

@@ -38,7 +38,9 @@ def factor_cosine_topk(item_factors, num_factors=None, topk=50, q_lo=0, q_hi=Non
     """Top-``topk`` most similar movies of every query movie ``q_lo <= q < q_hi``.
 
     :param item_factors: ``(num_items, num_factors)`` array, or the flat ``num_items*num_factors``
-        array ``cpp_ls.als`` returns together with ``num_factors``
+        array ``cpp_ls.als`` returns together with ``num_factors``; 1 to 160 factors (every rank
+        the exact ALS solvers train; 1 to 64 with ``MRB_SIM_KERNEL=dmma``)
+    :param topk: 1 to 56
     :return: ids ``int32[q, topk]`` (-1 padded), scores ``float64[q, topk]``, ``SimInfo``
     """
     M = numpy.ascontiguousarray(item_factors, dtype=numpy.double)
